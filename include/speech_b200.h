@@ -147,7 +147,6 @@ int sb_ctc_prefix_beam(const float* logp, const int* lens, int B, int T, int S, 
  *   sb_conv_relu_to_bct  C of the last layer -> (B, To, Co*Fo) f32 with ReLU (model.py:66-71)
  *   sb_conv_dtop         dY (B,To,Co*Fo) * (C>0) -> dC bf16 [M][Co]; db[c] += column sums
  *   sb_conv_col2im_relu  dA f32 [M][ldA] -> dC of the layer below (gather, masked by Pprev>0)
- *   sb_transpose_bf16    [R][C] -> [C][R] (weight-gradient operands)
  * ------------------------------------------------------------------------------------- */
 /* `mask_u8` (may be NULL): dropout keep-bytes (1 keep, 0 drop) of the activations involved, same
  * pixel-major channels-last layout as those activations; kept values are multiplied by `mscale`
@@ -162,8 +161,6 @@ int sb_conv_dtop(const float* dY, const float* C, const void* mask_u8, float msc
 int sb_conv_col2im_relu(const float* dA, long long ldA, const float* Pprev,
                         const void* maskprev_u8, float mscale, void* dCprev_bf16, float* db, int B,
                         int Ti, int Fi, int Ci, int kh, int kw, int stride, void* stream);
-int sb_transpose_bf16(const void* src, void* dst, long long R, int C, long long ld_src,
-                      long long ld_dst, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * Tail of the training step over flat fp32 buffers.
@@ -350,20 +347,9 @@ int sb_log_specgram(const short* pcm, const long long* offsets, const int* n_sam
 /* Developer hook (not part of the drop-in surface): device buffer of >= 64*16 uint64 receiving a
  * globaltimer timeline of CTA 0 for the next sb_gru_fwd launches; NULL disables. */
 int sb_debug_gru_timeline(void* dev_buffer);
-/* Developer hook, kernel selection of sb_gemm_bf16_tn (default 1|4): bit 0 = no 256-row
- * single-CTA tile variant, bit 1 = register-store epilogue instead of TMA stores, bit 2 = allow
- * the CTA-pair (tcgen05 cta_group::2) kernel. */
-int sb_debug_gemm_mt1(int force);
-int sb_debug_umma_mn(int lbo_bytes, int sbo_bytes, int kadv_bytes);
-/* Developer hook, GRU kernel selection / timing knobs (0 = defaults): 8 / 16 = never / always use
- * the transposed-accumulator K-split kernels, 32 = no K-split forward kernel, 64 / 128 = polling
- * mode of the grid barrier; 1 / 2 are timing ablations (results become wrong). */
-int sb_debug_gru_flags(int flags);
-/* Developer hook: enable (1, default) / disable (0) the K-split backward GRU kernel. */
-int sb_debug_gru_ksplit(int enable);
-/* Developer hook: set the preferred thread-block-cluster size (1, 2, 4 or 8) of the GRU kernels;
- * returns the cluster size the last GRU launch actually used (0 = query only, -1 = bad value). */
-int sb_debug_gru_cluster(int cluster_size);
+/* Developer hook, query only: with query = 0, returns the thread-block-cluster size the last
+ * sb_gru_fwd / sb_gru_bwd launch used (0 before the first one); any other argument returns -1. */
+int sb_debug_gru_cluster(int query);
 
 #ifdef __cplusplus
 }

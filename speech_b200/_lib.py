@@ -34,7 +34,6 @@ SIGNATURES = {
     "sb_conv_dtop": (_c_int, [_vp, _vp, _vp, _fl, _vp, _vp, _c_int, _c_int, _c_int, _c_int, _vp]),
     "sb_conv_col2im_relu": (_c_int, [_vp, _c_ll, _vp, _vp, _fl, _vp, _vp, _c_int, _c_int, _c_int,
                                      _c_int, _c_int, _c_int, _c_int, _vp]),
-    "sb_transpose_bf16": (_c_int, [_vp, _vp, _c_ll, _c_int, _c_ll, _c_ll, _vp]),
     "sb_sumsq_workspace_size": (_c_int, [ctypes.POINTER(_c_sz)]),
     "sb_sumsq": (_c_int, [_vp, _c_ll, _vp, _vp, _vp]),
     "sb_sgd_clip_step": (_c_int, [_vp, _vp, _vp, _vp, _c_ll, _vp, _fl, _fl, _fl, _vp]),
@@ -76,10 +75,6 @@ SIGNATURES = {
                                        _vp, _vp, _vp, _vp, _c_sz, _vp]),
     "sb_debug_gru_timeline": (_c_int, [_vp]),
     "sb_debug_gru_cluster": (_c_int, [_c_int]),
-    "sb_debug_gru_ksplit": (_c_int, [_c_int]),
-    "sb_debug_gru_flags": (_c_int, [_c_int]),
-    "sb_debug_gemm_mt1": (_c_int, [_c_int]),
-    "sb_debug_umma_mn": (_c_int, [_c_int, _c_int, _c_int]),
     "sb_edit_distance": (_c_ll, [_vp, _c_ll, _vp, _c_ll]),
     "sb_log_specgram": (_c_int, [_vp, _vp, _vp, _c_int, _c_int, _c_int, ctypes.c_double, _fl, _vp,
                                  _vp, _vp, _c_int, _vp]),

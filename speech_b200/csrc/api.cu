@@ -3,7 +3,7 @@
 
 #include "../../include/speech_b200.h"
 
-extern "C" int sb_version(void) { return 100; }
+extern "C" int sb_version(void) { return 101; }
 
 extern "C" const char* sb_status_string(int status) {
   switch (status) {

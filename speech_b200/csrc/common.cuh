@@ -240,12 +240,6 @@ SB_DEVINL unsigned int ld_acquire_gpu(const unsigned int* p) {
   asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
   return v;
 }
-SB_DEVINL unsigned int ld_relaxed_gpu(const unsigned int* p) {
-  unsigned int v;
-  asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-SB_DEVINL void fence_acq_rel_gpu() { asm volatile("fence.acq_rel.gpu;" ::: "memory"); }
 SB_DEVINL uint4 ld_cg_u4(const void* p) {
   uint4 v;
   asm volatile("ld.global.cg.v4.u32 {%0, %1, %2, %3}, [%4];"

@@ -12,7 +12,7 @@
 //   im2col matrix A[m][(i*kw + j)*Ci + ci] bf16 (K padded to a multiple of 8 with zeros); the
 //       weights are permuted to the same K order on the host side (40 K elements);
 //   conv = sb_gemm_bf16_tn(A, Wp) + bias  on tcgen05.
-// Backward: dC (pre-activation grad, bf16) -> dW = dC^T A (GEMM on transposed copies, split-K),
+// Backward: dC (pre-activation grad, bf16) -> dW^T = A^T dC (GEMM, both operands MN-major, split-K),
 //   dA = dC Wp (GEMM), col2im as a GATHER (each input pixel sums its <= ceil(kh/s)*ceil(kw/s)
 //   taps; no atomics) fused with the ReLU mask of the layer below.
 // All kernels here are HBM-bound elementwise/gather kernels (algorithmic bytes = one read of the
@@ -302,51 +302,6 @@ col2im_relu_generic_kernel(const float* __restrict__ dA, long long ldA,
     if (dbs[c] != 0.f) atomicAdd(db + c, dbs[c]);
 }
 
-// ---- bf16 matrix transpose [R][C] -> [C][ld_dst] ------------------------------------------------
-// 64x64 tiles, 32-bit (bf16x2) global accesses on both sides, padded shared tile.
-__global__ void __launch_bounds__(256)
-transpose_bf16_kernel(const bf16* __restrict__ src, bf16* __restrict__ dst, long long R, int C,
-                      long long ld_src, long long ld_dst) {
-  __shared__ unsigned short tile[64][66];
-  const long long r0 = (long long)blockIdx.x * 64;
-  const int c0 = blockIdx.y * 64;
-  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;   // 32 x 8
-  const unsigned short* s16 = reinterpret_cast<const unsigned short*>(src);
-  unsigned short* d16 = reinterpret_cast<unsigned short*>(dst);
-  const bool src_vec = ((ld_src & 1) == 0) && ((reinterpret_cast<uintptr_t>(src) & 3) == 0);
-  for (int rr = ty; rr < 64; rr += 8) {
-    const long long r = r0 + rr;
-    const int c = c0 + 2 * tx;
-    unsigned short a = 0, b = 0;
-    if (r < R) {
-      if (src_vec && c + 1 < C) {
-        const unsigned int u = *reinterpret_cast<const unsigned int*>(s16 + r * ld_src + c);
-        a = (unsigned short)(u & 0xffff); b = (unsigned short)(u >> 16);
-      } else {
-        if (c < C) a = s16[r * ld_src + c];
-        if (c + 1 < C) b = s16[r * ld_src + c + 1];
-      }
-    }
-    tile[rr][2 * tx] = a;
-    tile[rr][2 * tx + 1] = b;
-  }
-  __syncthreads();
-  const bool dst_vec = ((ld_dst & 1) == 0) && ((reinterpret_cast<uintptr_t>(dst) & 3) == 0);
-  for (int cc = ty; cc < 64; cc += 8) {
-    const int c = c0 + cc;
-    const long long r = r0 + 2 * tx;
-    if (c >= C) continue;
-    const unsigned short a = tile[2 * tx][cc], b = tile[2 * tx + 1][cc];
-    if (dst_vec && r + 1 < R) {
-      *reinterpret_cast<unsigned int*>(d16 + (long long)c * ld_dst + r) =
-          (unsigned int)a | ((unsigned int)b << 16);
-    } else {
-      if (r < R) d16[(long long)c * ld_dst + r] = a;
-      if (r + 1 < R) d16[(long long)c * ld_dst + r + 1] = b;
-    }
-  }
-}
-
 static int grid_for(long long total) {
   long long g = (total + 255) / 256;
   const long long cap = (long long)device_sm_count() * 16;
@@ -436,17 +391,5 @@ extern "C" int sb_conv_col2im_relu(const float* dA, long long ldA, const float* 
         Fi, Ci, kh, kw, stride, To, Fo);
 #undef SB_C2I
 #undef SB_C2I4
-  return cudaGetLastError() == cudaSuccess ? SB_OK : SB_ERR_CUDA;
-}
-
-extern "C" int sb_transpose_bf16(const void* src, void* dst, long long R, int C, long long ld_src,
-                                 long long ld_dst, void* stream_) {
-  if (!src || !dst || R <= 0 || C <= 0) return SB_ERR_INVALID;
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  dim3 grid((unsigned)((R + 63) / 64), (unsigned)((C + 63) / 64));
-  if (grid.y > 65535) return SB_ERR_UNSUPPORTED;
-  transpose_bf16_kernel<<<grid, 256, 0, stream>>>(reinterpret_cast<const bf16*>(src),
-                                                  reinterpret_cast<bf16*>(dst), R, C, ld_src,
-                                                  ld_dst);
   return cudaGetLastError() == cudaSuccess ? SB_OK : SB_ERR_CUDA;
 }

@@ -44,43 +44,37 @@ struct GemmParams {
 // units: 8 K-rows of 128 B per swizzle atom (SBO = 1024 B between atoms), the next 64 MN at
 // LBO = 8192 B (the next box).  One MMA (K = 16) spans two atoms; the next MMA starts 2048 B on.
 static constexpr int MN_BOX_BYTES = 64 * 64 * 2;
-static int g_mn_lbo = MN_BOX_BYTES, g_mn_sbo = 1024, g_mn_kadv = 2048;   // developer knobs
+static constexpr uint32_t MN_LBO = MN_BOX_BYTES, MN_SBO = 1024, MN_KADV = 2048;
 
-struct MnDesc { uint32_t lbo, sbo, kadv; };
-SB_DEVINL uint64_t umma_desc_sw128_mnmajor(uint32_t smem_addr, uint32_t lbo, uint32_t sbo) {
+SB_DEVINL uint64_t umma_desc_sw128_mnmajor(uint32_t smem_addr) {
   uint64_t d = 0;
   d |= (uint64_t)((smem_addr & 0x3FFFF) >> 4);
-  d |= (uint64_t)((lbo >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)((sbo >> 4) & 0x3FFF) << 32;
+  d |= (uint64_t)((MN_LBO >> 4) & 0x3FFF) << 16;
+  d |= (uint64_t)((MN_SBO >> 4) & 0x3FFF) << 32;
   d |= (uint64_t)1 << 46;
   d |= (uint64_t)2 << 61;
   return d;
 }
 
-// MT = number of 128-row MMA sub-tiles per CTA tile.  MT = 2 (256 x BN CTA tile) re-uses every B
-// tile for two MMAs: operand traffic per FLOP drops 1.5x at BN = 256 (the 128x256 tile measured
-// 12.4 TB/s of L2->SM reads with the tensor pipe only 55 % busy), at the price of a single
-// accumulator stage (all 512 TMEM columns hold one tile), so it is used for long-K GEMMs only.
-template <int BN, int MT>
+template <int BN>
 struct GemmCfg {
-  static constexpr int kStageBytes = (MT * BM + BN) * BK * 2;
+  static constexpr int kStageBytes = (BM + BN) * BK * 2;
   static constexpr int kStagesRaw = (200 * 1024) / kStageBytes;
   static constexpr int kStages = kStagesRaw > 8 ? 8 : kStagesRaw;
-  static constexpr int kAccStages = MT == 1 ? 2 : 1;
-  static constexpr int kTmemColsRaw = kAccStages * MT * BN;
+  static constexpr int kAccStages = 2;
+  static constexpr int kTmemColsRaw = kAccStages * BN;
   static constexpr int kTmemCols = kTmemColsRaw < 32 ? 32 : kTmemColsRaw;
   static constexpr int kStageOutBytes = 4 * 2 * 4096;   // 4 epilogue warps x 2 x [32 x 32] f32
   static constexpr int kSmemBytes =
       kStages * kStageBytes + kStageOutBytes + 1024 /*align*/ + 256 /*barriers*/;
 };
 
-template <int BN, int MT>
+template <int BN>
 __global__ void __launch_bounds__(192, 1)
 gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
                     const __grid_constant__ CUtensorMap tmap_b,
-                    const __grid_constant__ CUtensorMap tmap_c, const GemmParams p,
-                    const MnDesc mn) {
-  using Cfg = GemmCfg<BN, MT>;
+                    const __grid_constant__ CUtensorMap tmap_c, const GemmParams p) {
+  using Cfg = GemmCfg<BN>;
   constexpr int kStages = Cfg::kStages;
   constexpr int kAcc = Cfg::kAccStages;
   extern __shared__ uint8_t smem_raw[];
@@ -138,15 +132,15 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
         for (int kb = kb0; kb < kb1; ++kb) {
           mbar_wait(&empty_bar[stage], phase ^ 1);
           uint8_t* sa = tiles + stage * Cfg::kStageBytes;
-          uint8_t* sb_ = sa + MT * BM * BK * 2;
+          uint8_t* sb_ = sa + BM * BK * 2;
           mbar_expect_tx(&full_bar[stage], Cfg::kStageBytes);
           if (p.a_mn) {
 #pragma unroll
-            for (int b = 0; b < MT * BM / 64; ++b)
-              tma_load_2d(sa + b * MN_BOX_BYTES, &tmap_a, &full_bar[stage],
-                          m_blk * (MT * BM) + b * 64, kb * BK);
+            for (int b = 0; b < BM / 64; ++b)
+              tma_load_2d(sa + b * MN_BOX_BYTES, &tmap_a, &full_bar[stage], m_blk * BM + b * 64,
+                          kb * BK);
           } else {
-            tma_load_2d(sa, &tmap_a, &full_bar[stage], kb * BK, m_blk * (MT * BM));
+            tma_load_2d(sa, &tmap_a, &full_bar[stage], kb * BK, m_blk * BM);
           }
           if (p.b_mn) {
 #pragma unroll
@@ -164,8 +158,8 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
     // ===================== MMA issuer =====================
     const uint32_t idesc = umma_idesc_bf16_f32(BM, BN) | (p.a_mn ? (1u << 15) : 0u) |
                            (p.b_mn ? (1u << 16) : 0u);
-    const uint64_t a_step = p.a_mn ? (uint64_t)(mn.kadv >> 4) : 2u;
-    const uint64_t b_step = p.b_mn ? (uint64_t)(mn.kadv >> 4) : 2u;
+    const uint64_t a_step = p.a_mn ? (uint64_t)(MN_KADV >> 4) : 2u;
+    const uint64_t b_step = p.b_mn ? (uint64_t)(MN_KADV >> 4) : 2u;
     int stage = 0;
     uint32_t phase = 0;
     int acc = 0;
@@ -178,27 +172,21 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
       if (lane == 0) mbar_wait(&tempty_bar[acc], acc_phase ^ 1);
       __syncwarp();
       tc_fence_after_sync();
-      const uint32_t tmem_d = tmem_base + acc * (MT * BN);
+      const uint32_t tmem_d = tmem_base + acc * BN;
       for (int kb = kb0; kb < kb1; ++kb) {
         if (lane == 0) {
           mbar_wait(&full_bar[stage], phase);
           tc_fence_after_sync();
           const uint32_t sa = smem_u32(tiles + stage * Cfg::kStageBytes);
-          const uint32_t sb_ = sa + MT * BM * BK * 2;
-          const uint64_t db = p.b_mn ? umma_desc_sw128_mnmajor(sb_, mn.lbo, mn.sbo)
-                                     : umma_desc_sw128_kmajor(sb_);
+          const uint32_t sb_ = sa + BM * BK * 2;
+          const uint64_t da = p.a_mn ? umma_desc_sw128_mnmajor(sa) : umma_desc_sw128_kmajor(sa);
+          const uint64_t db = p.b_mn ? umma_desc_sw128_mnmajor(sb_) : umma_desc_sw128_kmajor(sb_);
 #pragma unroll
-          for (int mt = 0; mt < MT; ++mt) {
-            const uint64_t da = p.a_mn
-                                    ? umma_desc_sw128_mnmajor(sa + mt * BM * BK * 2, mn.lbo, mn.sbo)
-                                    : umma_desc_sw128_kmajor(sa + mt * BM * BK * 2);
-#pragma unroll
-            for (int k = 0; k < BK / 16; ++k) {
-              // K-major: advance 16 bf16 = 32 bytes along K inside the swizzle atom (+2 in the
-              // >>4 field); MN-major: 16 K-rows of 128 B = 2048 bytes
-              umma_bf16_ss(tmem_d + mt * BN, da + a_step * k, db + b_step * k, idesc,
-                           (kb > kb0 || k > 0) ? 1u : 0u);
-            }
+          for (int k = 0; k < BK / 16; ++k) {
+            // K-major: advance 16 bf16 = 32 bytes along K inside the swizzle atom (+2 in the
+            // >>4 field); MN-major: 16 K-rows of 128 B = 2048 bytes
+            umma_bf16_ss(tmem_d, da + a_step * k, db + b_step * k, idesc,
+                         (kb > kb0 || k > 0) ? 1u : 0u);
           }
           umma_commit(&empty_bar[stage]);  // frees the smem slot when these MMAs retire
           if (kb == kb1 - 1) umma_commit(&tfull_bar[acc]);
@@ -228,9 +216,7 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
       const bool has_k = kb0 < p.k_blocks_total;
       mbar_wait(&tfull_bar[acc], acc_phase);
       tc_fence_after_sync();
-#pragma unroll 1
-      for (int mt = 0; mt < MT; ++mt) {
-      const int m = m_blk * (MT * BM) + mt * BM + sub * 32 + lane;
+      const int m = m_blk * BM + sub * 32 + lane;
       bool row_ok = m < p.M;
       long long out_row = m;
       if (p.flags & SB_GEMM_ROW_REMAP) {
@@ -244,14 +230,12 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
 #pragma unroll 1
       for (int c = 0; c < BN / 32; ++c) {
         uint32_t v[32];
-        const uint32_t taddr =
-            tmem_base + ((uint32_t)(sub * 32) << 16) + acc * (MT * BN) + mt * BN + c * 32;
-        tmem_ld_32x32b_x32(taddr, v);
+        tmem_ld_32x32b_x32(tmem_base + ((uint32_t)(sub * 32) << 16) + acc * BN + c * 32, v);
         tmem_ld_wait();
         const int n0 = n_blk * BN + c * 32;
         if (p.tma_store) {
           // ---- coalesced path: registers -> swizzled smem tile -> one bulk tensor store ----
-          const int m0 = m_blk * (MT * BM) + mt * BM + sub * 32;
+          const int m0 = m_blk * BM + sub * 32;
           if (has_k && n0 < p.N && m0 < p.M) {      // warp-uniform
             uint8_t* buf = out_stage + ((warp - 2) * 2 + (out_slot & 1)) * 4096;
             if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
@@ -328,7 +312,6 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,
           }
         }
       }
-      }  // mt
       tc_fence_before_sync();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tempty_bar[acc]);
@@ -455,8 +438,7 @@ struct GemmPairCfg {
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1)
 gemm_bf16_tn_pair_kernel(const __grid_constant__ CUtensorMap tmap_a,
                          const __grid_constant__ CUtensorMap tmap_b,
-                         const __grid_constant__ CUtensorMap tmap_c, const GemmParams p,
-                         const MnDesc mn) {
+                         const __grid_constant__ CUtensorMap tmap_c, const GemmParams p) {
   using Cfg = GemmPairCfg;
   constexpr int kStages = Cfg::kStages;
   constexpr int BN = Cfg::BN;
@@ -546,8 +528,8 @@ gemm_bf16_tn_pair_kernel(const __grid_constant__ CUtensorMap tmap_a,
     if (rank == 0) {
       const uint32_t idesc = umma_idesc_bf16_f32(2 * BM, BN) | (p.a_mn ? (1u << 15) : 0u) |
                              (p.b_mn ? (1u << 16) : 0u);
-      const uint64_t a_step = p.a_mn ? (uint64_t)(mn.kadv >> 4) : 2u;
-      const uint64_t b_step = p.b_mn ? (uint64_t)(mn.kadv >> 4) : 2u;
+      const uint64_t a_step = p.a_mn ? (uint64_t)(MN_KADV >> 4) : 2u;
+      const uint64_t b_step = p.b_mn ? (uint64_t)(MN_KADV >> 4) : 2u;
       int stage = 0;
       uint32_t phase = 0;
       int acc = 0;
@@ -562,9 +544,8 @@ gemm_bf16_tn_pair_kernel(const __grid_constant__ CUtensorMap tmap_a,
             mbar_wait(&full_bar[stage], phase);
             tc_fence_after_sync();
             const uint32_t sa = smem_u32(tiles + stage * Cfg::kStageBytes);
-            const uint64_t da = p.a_mn ? umma_desc_sw128_mnmajor(sa, mn.lbo, mn.sbo)
-                                       : umma_desc_sw128_kmajor(sa);
-            const uint64_t db = p.b_mn ? umma_desc_sw128_mnmajor(sa + BM * BK * 2, mn.lbo, mn.sbo)
+            const uint64_t da = p.a_mn ? umma_desc_sw128_mnmajor(sa) : umma_desc_sw128_kmajor(sa);
+            const uint64_t db = p.b_mn ? umma_desc_sw128_mnmajor(sa + BM * BK * 2)
                                        : umma_desc_sw128_kmajor(sa + BM * BK * 2);
 #pragma unroll
             for (int k = 0; k < BK / 16; ++k)
@@ -720,15 +701,13 @@ static int make_tmap_f32_c(CUtensorMap* map, float* base, long long rows, long l
   return r == CUDA_SUCCESS ? SB_OK : SB_ERR_CUDA;
 }
 
-static int g_gemm_tma_store = 1;
-
-template <int BN, int MT>
+template <int BN>
 static int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, GemmParams p,
                        cudaStream_t stream) {
-  using Cfg = GemmCfg<BN, MT>;
+  using Cfg = GemmCfg<BN>;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(gemm_bf16_tn_kernel<BN, MT>,
+    cudaError_t e = cudaFuncSetAttribute(gemm_bf16_tn_kernel<BN>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          Cfg::kSmemBytes);
     if (e != cudaSuccess) return SB_ERR_CUDA;
@@ -740,12 +719,11 @@ static int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, GemmParams 
   if (grid > total) grid = total;
   CUtensorMap tc = ta;   // placeholder when the register epilogue is used
   p.tma_store = 0;
-  if (g_gemm_tma_store && !(p.flags & SB_GEMM_ROW_REMAP) && (p.ldc & 3) == 0 &&
+  if (!(p.flags & SB_GEMM_ROW_REMAP) && (p.ldc & 3) == 0 &&
       (reinterpret_cast<uintptr_t>(p.C) & 15) == 0) {
     if (make_tmap_f32_c(&tc, p.C, p.M, p.N, p.ldc) == SB_OK) p.tma_store = 1;
   }
-  const MnDesc mn = {(uint32_t)g_mn_lbo, (uint32_t)g_mn_sbo, (uint32_t)g_mn_kadv};
-  gemm_bf16_tn_kernel<BN, MT><<<grid, 192, Cfg::kSmemBytes, stream>>>(ta, tb, tc, p, mn);
+  gemm_bf16_tn_kernel<BN><<<grid, 192, Cfg::kSmemBytes, stream>>>(ta, tb, tc, p);
   return cudaGetLastError() == cudaSuccess ? SB_OK : SB_ERR_CUDA;
 }
 
@@ -770,9 +748,6 @@ static int pick_wave_filling_split(long long tiles, int units, int k_blocks) {
   return best_split;
 }
 
-static int g_gemm_force_mt1 = 1;   // the 256-row CTA tile measured slower (epilogue not overlapped)
-static int g_gemm_pair = 1;        // CTA-pair (cta_group::2) kernel for the large tiles
-
 // CTA-pair launch: needs the TMA-store epilogue (no row remap, 16-byte aligned C rows)
 static int launch_gemm_pair(const CUtensorMap& ta, const CUtensorMap& tb, GemmParams p,
                             cudaStream_t stream) {
@@ -793,33 +768,13 @@ static int launch_gemm_pair(const CUtensorMap& ta, const CUtensorMap& tb, GemmPa
   CUtensorMap tc;
   if (make_tmap_f32_c(&tc, p.C, p.M, p.N, p.ldc) != SB_OK) return SB_ERR_CUDA;
   p.tma_store = 1;
-  const MnDesc mn = {(uint32_t)g_mn_lbo, (uint32_t)g_mn_sbo, (uint32_t)g_mn_kadv};
-  gemm_bf16_tn_pair_kernel<<<2 * pairs, 192, Cfg::kSmemBytes, stream>>>(ta, tb, tc, p, mn);
+  gemm_bf16_tn_pair_kernel<<<2 * pairs, 192, Cfg::kSmemBytes, stream>>>(ta, tb, tc, p);
   return cudaGetLastError() == cudaSuccess ? SB_OK : SB_ERR_CUDA;
 }
 
 }  // namespace sb
 
 using namespace sb;
-
-// developer hook (kernel selection); the default state is force = 1 | 4
-// developer hook: override the MN-major descriptor fields (bytes); 0 keeps a field
-extern "C" int sb_debug_umma_mn(int lbo, int sbo, int kadv) {
-  if (lbo > 0) sb::g_mn_lbo = lbo;
-  if (sbo > 0) sb::g_mn_sbo = sbo;
-  if (kadv > 0) sb::g_mn_kadv = kadv;
-  return SB_OK;
-}
-
-extern "C" int sb_debug_gemm_mt1(int force) {
-  // bit 0: 1 = 128-row CTA tiles only (default), 0 = allow the 256-row variant
-  // bit 1: 1 = disable the TMA-store epilogue (register stores)
-  // bit 2: 1 = CTA-pair (cta_group::2) kernel for 256-wide tiles
-  sb::g_gemm_force_mt1 = force & 1;
-  sb::g_gemm_tma_store = (force & 2) ? 0 : 1;
-  sb::g_gemm_pair = (force & 4) ? 1 : 0;
-  return SB_OK;
-}
 
 extern "C" int sb_gemm_bf16_tn(const void* A, long long lda, const void* B, long long ldb, float* C,
                                long long ldc, const float* bias, int M, int N, int K, int flags,
@@ -859,13 +814,7 @@ extern "C" int sb_gemm_bf16_tn(const void* A, long long lda, const void* B, long
     const long long tiles256 = (long long)p.m_tiles * ((N + 255) / 256) * split_k;
     bn = (tiles256 >= sms || N > 2048) ? 256 : 128;
   }
-  // 256-row CTA tiles when the GEMM is long (K >= 1024) and still leaves >= 3 waves of tiles
-  int mt = 1;
-  if (bn == 256 && K >= 1024 && split_k == 1 && !g_gemm_force_mt1) {
-    const long long tiles2 = (long long)((M + 2 * BM - 1) / (2 * BM)) * ((N + 255) / 256);
-    if (tiles2 >= 3LL * sms) mt = 2;
-  }
-  if (N > 128 && g_gemm_pair && g_gemm_tma_store && !(flags & SB_GEMM_ROW_REMAP) &&
+  if (N > 128 && !(flags & SB_GEMM_ROW_REMAP) &&
       (ldc & 3) == 0 && (reinterpret_cast<uintptr_t>(C) & 15) == 0) {
     const long long pair_tiles = (long long)((M + 2 * BM - 1) / (2 * BM)) * ((N + 255) / 256);
     const int pairs = sms / 2;
@@ -885,20 +834,18 @@ extern "C" int sb_gemm_bf16_tn(const void* A, long long lda, const void* B, long
       return launch_gemm_pair(pa, pb, p, stream);
     }
   }
-  p.m_tiles = (M + mt * BM - 1) / (mt * BM);
   if (flags & SB_GEMM_ACCUMULATE)
     p.split_k = pick_wave_filling_split((long long)p.m_tiles * ((N + bn - 1) / bn), sms,
                                         p.k_blocks_total);
   CUtensorMap ta, tb;
-  int rc = tmap_a(&ta, mt * BM);
+  int rc = tmap_a(&ta, BM);
   if (rc != SB_OK) return rc;
   rc = tmap_b(&tb, bn);
   if (rc != SB_OK) return rc;
-  if (mt == 2) return launch_gemm<256, 2>(ta, tb, p, stream);
   switch (bn) {
-    case 32: return launch_gemm<32, 1>(ta, tb, p, stream);
-    case 64: return launch_gemm<64, 1>(ta, tb, p, stream);
-    case 128: return launch_gemm<128, 1>(ta, tb, p, stream);
-    default: return launch_gemm<256, 1>(ta, tb, p, stream);
+    case 32: return launch_gemm<32>(ta, tb, p, stream);
+    case 64: return launch_gemm<64>(ta, tb, p, stream);
+    case 128: return launch_gemm<128>(ta, tb, p, stream);
+    default: return launch_gemm<256>(ta, tb, p, stream);
   }
 }

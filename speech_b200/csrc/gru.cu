@@ -6,12 +6,12 @@
 // (speech/models/transducer_model.py:23-26,68).
 //
 // The time-batched input projection gi = X W_ih^T + b_ih is done for all T at once by
-// sb_gemm_bf16_tn; these kernels run the T-serial part.  One cooperative launch per layer covers
-// BOTH directions:
+// sb_gemm_bf16_tn; these kernels run the T-serial part.  One launch per layer covers BOTH
+// directions:
 //   * CTA c of direction d owns 16 hidden units j0..j0+15: its 48 rows of W_hh (r,z,n) stay
 //     resident in shared memory (bf16, UMMA K-major SWIZZLE_128B chunks) for all T steps;
 //   * per step every CTA needs ALL of h_{t-1} (bf16, written by the CTAs of its direction in the
-//     previous step).  CTAs form thread-block clusters of up to 8; each CTA fetches 1/CS of the
+//     previous step).  CTAs form thread-block clusters of up to 4; each CTA fetches 1/CS of the
 //     [Bp x 64] chunks with TMA and MULTICASTS them into the shared memory of all CTAs of its
 //     cluster, so L2 is read once per cluster instead of once per CTA (the un-multicast version
 //     was bound by 64 SMs hammering the same L2 lines: 4 us of a 13 us step);
@@ -20,7 +20,7 @@
 //   * 8 epilogue warps (thread = TMEM lane = batch row, 8 hidden units each) read the
 //     accumulators with tcgen05.ld, apply the gate math in fp32 (h_{t-1} of the thread's own units
 //     stays in registers across steps), publish the bf16 h_t, arrive on the per-direction grid
-//     barrier, and only then write the fp32 state / transposed copy / saved gates;
+//     barrier, and only then write the fp32 state / saved gates;
 //   * the grid barrier is one red.release.gpu + ld.acquire.gpu polling on a global counter.
 // The backward kernel has the same structure with W_hh^T resident (16 rows x 3H) and the
 // all-gather over the pre-activation gradients dgh_t (batch x 3H).
@@ -50,12 +50,10 @@ struct GruFwdParams {
   const float* bhh;    // [ndir][3H]
   float* y;            // [T*Bp][ndir*H]   h_t fp32
   bf16* xn;            // [T*Bp][ndir*H]   h_t bf16 (operand of the next projection)
-  bf16* xnT;           // [ndir*H][(T+2)*Bp] h_t bf16 transposed, column (t+1)*Bp+b ; may be null
   float* gates;        // [T*Bp][ndir][4][H] saved r,z,n,hn for backward ; may be null
   unsigned int* barrier;  // [ndir] zero-initialised counters
   unsigned long long* dbg;  // optional timeline (CTA 0): [step][16] globaltimer stamps, or null
   int T, Bp, H, ndir, ring, gc;   // ring: slots (groups of gc chunks) in shared memory
-  int ablate;          // developer knobs: see sb_debug_gru_flags
 };
 
 struct GruBwdParams {
@@ -71,7 +69,6 @@ struct GruBwdParams {
   unsigned int* barrier;  // [ndir]
   unsigned long long* dbg;
   int T, Bp, H, ndir, ring, gc;
-  int ablate;          // developer knobs (polling mode bits 64 / 128)
 };
 
 SB_DEVINL unsigned long long gtime() {
@@ -86,25 +83,14 @@ SB_DEVINL unsigned long long gtime() {
 
 // ---- per-direction grid barrier ------------------------------------------------------------
 SB_DEVINL void grid_arrive(unsigned int* ctr) { red_release_gpu_add(ctr, 1u); }
-// Polling modes of the grid barrier (developer knob sb_debug_gru_flags bits 64 / 128):
-//   0   : ld.acquire.gpu per poll (its implied fence throttles the poll rate)
-//   64  : ld.relaxed.gpu + nanosleep per poll, one fence.acq_rel.gpu when the count is complete
-//   128 : ld.relaxed.gpu + nanosleep per poll, no fence (the TMA reads that follow go to L2)
-// (Un-throttled relaxed polling was measured SLOWER, 7.8 vs 7.3 us/step: the tight spin of 128
-// pollers on the counter's L2 line delays the arriving reductions.)
-SB_DEVINL void grid_wait(const unsigned int* ctr, unsigned int target, int mode = 0) {
+// One ld.acquire.gpu per poll: its implied fence throttles the poll rate.  (Relaxed polling, with
+// or without nanosleep, was measured SLOWER, 7.8 vs 7.3 us/step: the tight spin of 128 pollers on
+// the counter's L2 line delays the arriving reductions.)
+SB_DEVINL void grid_wait(const unsigned int* ctr, unsigned int target) {
   unsigned int spins = 0;
-  if (mode == 0) {
-    while (ld_acquire_gpu(ctr) < target) {
-      if (++spins > SB_SPIN_LIMIT) __trap();
-    }
-    return;
-  }
-  while (ld_relaxed_gpu(ctr) < target) {
-    __nanosleep(64);
+  while (ld_acquire_gpu(ctr) < target) {
     if (++spins > SB_SPIN_LIMIT) __trap();
   }
-  if (mode & 64) fence_acq_rel_gpu();
 }
 SB_DEVINL void epi_barrier() { asm volatile("bar.sync 1, %0;" ::"n"(GRU_EPI) : "memory"); }
 
@@ -285,7 +271,6 @@ gru_fwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
   const GruSmem s = carve(smem_raw, ring_bytes, wbytes);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int D = p.ndir * H;
-  const long long ldT = (long long)(T + 2) * Bp;
   const CUtensorMap* tm = dir == 0 ? &tm_d0 : &tm_d1;
   const uint32_t crank = cluster_rank(), csize = cluster_size();
 
@@ -408,7 +393,7 @@ gru_fwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
         // critical path: only the bf16 h_t that the other CTAs gather next step
         *reinterpret_cast<uint4*>(p.xn + m * D + dir * H + ju) = pack8(hprev);
         if (tid == 0) GRU_STAMP(5);
-        if (!(p.ablate & 1)) fence_proxy_async_global();   // generic writes -> other CTAs' TMA reads
+        fence_proxy_async_global();   // generic writes -> other CTAs' TMA reads
         if (tid == 0) GRU_STAMP(6);
       }
       epi_barrier();
@@ -417,14 +402,9 @@ gru_fwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
         grid_arrive(ctr);          // release: cumulative over the CTA's writes ordered by bar.sync
         GRU_STAMP(9);
       }
-      // off the critical path: fp32 state, transposed copy, saved gates
-      if (active && !(p.ablate & 2)) {
+      // off the critical path: fp32 state, saved gates
+      if (active) {
         st8(p.y + m * D + dir * H + ju, hprev);
-        if (p.xnT) {
-          bf16* xt = p.xnT + (long long)(dir * H + ju) * ldT + (long long)(t + 1) * Bp + row;
-#pragma unroll
-          for (int jj = 0; jj < GRU_UPT; ++jj) st_stream_bf16(xt + jj * ldT, hprev[jj]);
-        }
         if (p.gates) {
           float* go = p.gates + ((m * p.ndir + dir) * 4) * H + ju;
           st8(go, rr);
@@ -780,7 +760,7 @@ gru_bwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
   if (warp == 9) {
     if (lane == 0) {
       for (int step = 0; step + 1 < T; ++step) {
-        grid_wait(ctr, (unsigned int)nC * (step + 1), p.ablate & 192);   // dgh of this step is complete
+        grid_wait(ctr, (unsigned int)nC * (step + 1));   // dgh of this step is complete
         for (int g = 0; g < ngroups; ++g) {
           mbar_expect_tx(&full[g], (uint32_t)(stride * gc));
           for (int i = 0; i < gc; ++i) {
@@ -1061,7 +1041,7 @@ gru_fwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
       for (int step = 1; step < T; ++step) {
         const int t = dir == 0 ? step : (T - 1 - step);
         const int tp = dir == 0 ? t - 1 : t + 1;
-        grid_wait(ctr, (unsigned int)nC * step, p.ablate & 192);   // all CTAs published h_{tp}
+        grid_wait(ctr, (unsigned int)nC * step);   // all CTAs published h_{tp}
         GRU_STAMP(0);
         if (p.dbg && step == 21) p.dbg[1024 + 256 + blockIdx.x] = gtime();   // skew probe
         mbar_expect_tx(full, (uint32_t)(stride * nchunks));
@@ -1245,10 +1225,7 @@ gru_fwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
 // =============================================================================================
 template <int UPT>
 SB_DEVINL void ldu(const float* p, float (&v)[UPT]) {
-  if constexpr (UPT == 4) {
-    const float4 a = __ldcs(reinterpret_cast<const float4*>(p));
-    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w;
-  } else if constexpr (UPT == 2) {
+  if constexpr (UPT == 2) {
     const float2 a = __ldcs(reinterpret_cast<const float2*>(p));
     v[0] = a.x; v[1] = a.y;
   } else {
@@ -1257,15 +1234,12 @@ SB_DEVINL void ldu(const float* p, float (&v)[UPT]) {
 }
 template <int UPT>
 SB_DEVINL void stu(float* p, const float (&v)[UPT]) {
-  if constexpr (UPT == 4) __stcs(reinterpret_cast<float4*>(p), make_float4(v[0], v[1], v[2], v[3]));
-  else if constexpr (UPT == 2) __stcs(reinterpret_cast<float2*>(p), make_float2(v[0], v[1]));
+  if constexpr (UPT == 2) __stcs(reinterpret_cast<float2*>(p), make_float2(v[0], v[1]));
   else __stcs(p, v[0]);
 }
 template <int UPT>
 SB_DEVINL void st_bf16u(bf16* p, const float (&v)[UPT]) {
-  if constexpr (UPT == 4) {
-    *reinterpret_cast<uint2*>(p) = make_uint2(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]));
-  } else if constexpr (UPT == 2) {
+  if constexpr (UPT == 2) {
     *reinterpret_cast<uint32_t*>(p) = pack_bf16x2(v[0], v[1]);
   } else {
     *p = __float2bfloat16_rn(v[0]);
@@ -1358,7 +1332,7 @@ gru_fwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
       for (int step = 1; step < T; ++step) {
         const int t = dir == 0 ? step : (T - 1 - step);
         const int tp = dir == 0 ? t - 1 : t + 1;
-        grid_wait(ctr, (unsigned int)nC * step, p.ablate & 192);   // all CTAs published h_{tp}
+        grid_wait(ctr, (unsigned int)nC * step);   // all CTAs published h_{tp}
         GRU_STAMP(0);
         if (p.dbg && step == 21) p.dbg[1024 + 256 + blockIdx.x] = gtime();   // skew probe
         mbar_expect_tx(full, (uint32_t)(stride * nchunks));
@@ -1549,9 +1523,7 @@ gru_fwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
 // =============================================================================================
 template <int UPT>
 SB_DEVINL void st_stream_bf16u(bf16* p, const float (&v)[UPT]) {
-  if constexpr (UPT == 4) {
-    __stcs(reinterpret_cast<uint2*>(p), make_uint2(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3])));
-  } else if constexpr (UPT == 2) {
+  if constexpr (UPT == 2) {
     __stcs(reinterpret_cast<unsigned int*>(p), pack_bf16x2(v[0], v[1]));
   } else {
     st_stream_bf16(p, v[0]);
@@ -1640,7 +1612,7 @@ gru_bwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
   if (warp == 9) {
     if (lane == 0) {
       for (int step = 0; step + 1 < T; ++step) {
-        grid_wait(ctr, (unsigned int)nC * (step + 1), p.ablate & 192);   // dgh of this step is complete
+        grid_wait(ctr, (unsigned int)nC * (step + 1));   // dgh of this step is complete
         GRU_STAMP(0);
         for (int g = 0; g < ngroups; ++g) {
           mbar_expect_tx(&full[g], (uint32_t)(stride * gc));
@@ -1856,75 +1828,23 @@ static int gru_ring_slots(int wbytes, int Bp, int nchunks, int* gc_out, size_t* 
   return ring;
 }
 
-static int g_gru_cluster = 4;   // preferred cluster size (developer knob: sb_debug_gru_cluster)
 static int g_gru_last_cluster = 0;
-
-static int gru_cluster_size(int nC) {
-  int cs = g_gru_cluster;
-  while (cs > 1 && (nC % cs) != 0) cs >>= 1;
-  return cs < 1 ? 1 : cs;
-}
-
-static int gru_launch(const void* kernel, int grid, int cs, size_t smem, void** args,
-                      cudaStream_t stream) {
-  if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) !=
-      cudaSuccess)
-    return SB_ERR_CUDA;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(GRU_THREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attrs[2];
-  attrs[0].id = cudaLaunchAttributeCooperative;
-  attrs[0].val.cooperative = 1;
-  attrs[1].id = cudaLaunchAttributeClusterDimension;
-  attrs[1].val.clusterDim.x = cs;
-  attrs[1].val.clusterDim.y = 1;
-  attrs[1].val.clusterDim.z = 1;
-  cfg.attrs = attrs;
-  cfg.numAttrs = 2;
-  // all CTAs must be co-resident (grid barrier): shrink the cluster until the grid fits
-  if (cs > 1 &&
-      cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 0) != cudaSuccess)
-    cudaGetLastError();
-  for (; cs >= 1; cs >>= 1) {
-    attrs[1].val.clusterDim.x = cs;
-    int nclusters = 0;
-    if (cs > 1) {
-      if (cudaOccupancyMaxActiveClusters(&nclusters, kernel, &cfg) != cudaSuccess) {
-        cudaGetLastError();
-        continue;
-      }
-      if (nclusters * cs < grid) continue;
-    }
-    if (cudaLaunchKernelExC(&cfg, kernel, args) == cudaSuccess) {
-      g_gru_last_cluster = cs;
-      return SB_OK;
-    }
-    cudaGetLastError();
-  }
-  return SB_ERR_CUDA;
-}
-
 static unsigned long long* g_gru_dbg = nullptr;
-static int g_gru_ablate = 0;
-static int g_gru_ksplit = 1;   // developer knob: 0 disables the K-split backward kernel
 
 // Which K-split flavour: the transposed-accumulator kernels (gru_*_kt_kernel) win while the batch
 // is small.  Measured us/step at H = 1024 (kt | ks): forward 3.8 | 4.8 at 8 rows, 4.3 | 4.9 at 16,
 // 5.3 | 5.4 at 32, 7.9 | 7.1 at 64; backward 4.6 | 5.3 at 8, 5.4 | 5.4 at 16, 6.2 | 5.8 at 32,
-// 8.3 | 7.8 at 64.  Developer knob (sb_debug_gru_flags): 16 forces them, 8 disables them.
-static bool gru_use_kt(int Bp, bool backward) {
-  if (g_gru_ablate & 8) return false;
-  if (g_gru_ablate & 16) return true;
-  return Bp <= (backward ? 8 : 32);
-}
+// 8.3 | 7.8 at 64.
+static bool gru_use_kt(int Bp, bool backward) { return Bp <= (backward ? 8 : 32); }
 
-// cooperative launch with EXACTLY the given cluster size; fails if the grid is not co-resident
-static int gru_launch_exact(const void* kernel, int grid, int cs, size_t smem, void** args,
-                            cudaStream_t stream) {
+// Every GRU kernel synchronises each direction through a grid barrier in global memory, so the
+// whole grid must be resident at once.  Launches are not flagged cooperative: co-residency is
+// proven with the occupancy API (one CTA per SM, grid <= resident capacity), and every spin-wait
+// in the kernels is bounded.  The cluster size starts at cs_pref and halves while it does not
+// divide the nC CTAs of a direction or the grid does not fit, down to cs_min; SB_ERR_UNSUPPORTED
+// when no size fits, so that the caller can fall back to another kernel.
+static int gru_launch(const void* kernel, int grid, int nC, int cs_pref, int cs_min, size_t smem,
+                      void** args, cudaStream_t stream) {
   if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) !=
       cudaSuccess) {
     cudaGetLastError();
@@ -1936,29 +1856,42 @@ static int gru_launch_exact(const void* kernel, int grid, int cs, size_t smem, v
   cfg.blockDim = dim3(GRU_THREADS);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
-  // Clustered launches are NOT flagged cooperative: co-residency of the whole grid is established
-  // by the occupancy query below (1 CTA per SM, grid <= resident capacity), every spin-wait in
-  // the kernels is bounded, and Nsight Compute cannot replay cooperative+cluster launches.
-  cudaLaunchAttribute attrs[1];
-  attrs[0].id = cudaLaunchAttributeClusterDimension;
-  attrs[0].val.clusterDim.x = cs;
-  attrs[0].val.clusterDim.y = 1;
-  attrs[0].val.clusterDim.z = 1;
-  cfg.attrs = attrs;
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeClusterDimension;
+  attr.val.clusterDim.y = 1;
+  attr.val.clusterDim.z = 1;
+  cfg.attrs = &attr;
   cfg.numAttrs = 1;
-  int nclusters = 0;
-  if (cudaOccupancyMaxActiveClusters(&nclusters, kernel, &cfg) != cudaSuccess ||
-      nclusters * cs < grid) {
-    cudaGetLastError();
-    return SB_ERR_UNSUPPORTED;
+  for (int cs = cs_pref; cs >= cs_min; cs >>= 1) {
+    if (nC % cs != 0) continue;
+    attr.val.clusterDim.x = cs;
+    int resident = 0;
+    cudaError_t e;
+    if (cs > 1) {
+      e = cudaOccupancyMaxActiveClusters(&resident, kernel, &cfg);
+      resident *= cs;
+    } else {
+      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kernel, GRU_THREADS, smem);
+      resident *= device_sm_count();
+    }
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      continue;
+    }
+    if (resident < grid) continue;
+    if (cudaLaunchKernelExC(&cfg, kernel, args) != cudaSuccess) {
+      cudaGetLastError();
+      return SB_ERR_CUDA;
+    }
+    g_gru_last_cluster = cs;
+    return SB_OK;
   }
-  if (cudaLaunchKernelExC(&cfg, kernel, args) != cudaSuccess) {
-    cudaGetLastError();
-    return SB_ERR_CUDA;
-  }
-  g_gru_last_cluster = cs;
-  return SB_OK;
+  return SB_ERR_UNSUPPORTED;
 }
+
+// workspace of one recurrence launch: [0,1024) the per-direction grid-barrier words, then the
+// exchange buffers of the backward kernels
+static constexpr size_t GRU_WS_COUNTERS = 1024;
 
 }  // namespace sb
 
@@ -1969,25 +1902,8 @@ extern "C" int sb_debug_gru_timeline(void* dev_buffer) {
   sb::g_gru_dbg = reinterpret_cast<unsigned long long*>(dev_buffer);
   return SB_OK;
 }
-// developer knobs: 1 / 2: gru_fwd_kernel without the proxy fence / the off-path stores (timing
-// only: results become wrong); 8 / 16: never / always use the transposed-accumulator K-split
-// kernels (default: by batch size, see gru_use_kt); 32: disable the K-split forward kernels;
-// 64 / 128: polling mode of the grid barrier in the K-split kernels (see grid_wait)
-extern "C" int sb_debug_gru_flags(int flags) {
-  sb::g_gru_ablate = flags;
-  return SB_OK;
-}
-extern "C" int sb_debug_gru_ksplit(int enable) {
-  sb::g_gru_ksplit = enable ? 1 : 0;
-  return SB_OK;
-}
-extern "C" int sb_debug_gru_cluster(int cluster_size) {
-  // cluster_size 0 queries: returns the cluster size the last GRU launch actually used
-  if (cluster_size == 0) return sb::g_gru_last_cluster;
-  if (cluster_size != 1 && cluster_size != 2 && cluster_size != 4 && cluster_size != 8)
-    return -1;
-  sb::g_gru_cluster = cluster_size;
-  return sb::g_gru_last_cluster;
+extern "C" int sb_debug_gru_cluster(int query) {
+  return query == 0 ? sb::g_gru_last_cluster : -1;
 }
 
 static int gru_check(int T, int Bp, int H, int ndir) {
@@ -1997,17 +1913,10 @@ static int gru_check(int T, int Bp, int H, int ndir) {
   return SB_OK;
 }
 
-// workspace of one recurrence launch: [0,1024) the per-direction grid-barrier words, then the
-// exchange buffers of the backward kernels
-static size_t gru_ws_counters_bytes(int ndir) {
-  (void)ndir;
-  return 1024;
-}
-
 extern "C" int sb_gru_fwd_workspace_size(int Bp, int H, int ndir, size_t* bytes) {
   if (!bytes || Bp <= 0 || H <= 0 || (ndir != 1 && ndir != 2)) return SB_ERR_INVALID;
   (void)Bp;
-  *bytes = gru_ws_counters_bytes(ndir);      // the forward kernels exchange h_t through xn itself
+  *bytes = GRU_WS_COUNTERS;      // the forward kernels exchange h_t through xn itself
   return SB_OK;
 }
 
@@ -2034,16 +1943,16 @@ extern "C" int sb_gru_fwd(const float* gi, const void* whh_bf16, const float* bh
   if (ring < 0) return SB_ERR_UNSUPPORTED;
 
   // ---- preferred: K-split over 4-CTA clusters (H % 256 == 0, batch rows <= 64) ----
-  if (!(g_gru_ablate & 32) && H % 256 == 0 && nC % KS == 0 && Bp <= 64) {
+  if (H % 256 == 0 && nC % KS == 0 && Bp <= 64) {
     const int nq = H / KS / 64;
     const size_t ks_smem = (size_t)nq * Bp * 128 + (size_t)nq * 192 * 128 +
                            (size_t)2 * KS * Bp * 48 * 4 + 1024 + 512;
     if (ks_smem <= 227 * 1024) {
       GruFwdParams q;
       q.gi = gi; q.whh = reinterpret_cast<const bf16*>(whh_bf16); q.bhh = bhh; q.y = y;
-      q.xn = reinterpret_cast<bf16*>(xn_bf16); q.xnT = nullptr; q.gates = gates;
+      q.xn = reinterpret_cast<bf16*>(xn_bf16); q.gates = gates;
       q.barrier = barrier; q.T = T; q.Bp = Bp; q.H = H; q.ndir = ndir;
-      q.dbg = g_gru_dbg; q.ablate = g_gru_ablate & 192; q.ring = nq; q.gc = 1;
+      q.dbg = g_gru_dbg; q.ring = nq; q.gc = 1;
       CUtensorMap tq[2];
       for (int d = 0; d < 2; ++d) {
         const int dd = d < ndir ? d : 0;
@@ -2055,13 +1964,12 @@ extern "C" int sb_gru_fwd(const float* gi, const void* whh_bf16, const float* bh
       const size_t kt_smem = (size_t)nq * Bp * 128 + (size_t)nq * 192 * 128 +
                              (size_t)(2 * KS - 1) * 48 * (Bp + 4) * 4 + 1024 + 512;
       if (gru_use_kt(Bp, false) && kt_smem <= 227 * 1024) {
-        const void* kt = Bp > 32   ? (const void*)gru_fwd_kt_kernel<4>
-                         : Bp > 16 ? (const void*)gru_fwd_kt_kernel<2>
-                                   : (const void*)gru_fwd_kt_kernel<1>;
-        rc = gru_launch_exact(kt, ndir * nC, KS, kt_smem, kargs, stream);
+        const void* kt = Bp > 16 ? (const void*)gru_fwd_kt_kernel<2>
+                                 : (const void*)gru_fwd_kt_kernel<1>;
+        rc = gru_launch(kt, ndir * nC, nC, KS, KS, kt_smem, kargs, stream);
         if (rc == SB_OK) return SB_OK;
       }
-      rc = gru_launch_exact((const void*)gru_fwd_ks_kernel, ndir * nC, KS, ks_smem, kargs, stream);
+      rc = gru_launch((const void*)gru_fwd_ks_kernel, ndir * nC, nC, KS, KS, ks_smem, kargs, stream);
       if (rc == SB_OK) return SB_OK;
     }
   }
@@ -2069,10 +1977,9 @@ extern "C" int sb_gru_fwd(const float* gi, const void* whh_bf16, const float* bh
   // ---- every other shape: each CTA gathers all of h_{t-1} (tensor-map TMA, cluster multicast) ----
   GruFwdParams p;
   p.gi = gi; p.whh = reinterpret_cast<const bf16*>(whh_bf16); p.bhh = bhh; p.y = y;
-  p.xn = reinterpret_cast<bf16*>(xn_bf16); p.xnT = nullptr;
+  p.xn = reinterpret_cast<bf16*>(xn_bf16);
   p.gates = gates; p.barrier = barrier; p.T = T; p.Bp = Bp; p.H = H; p.ndir = ndir;
   p.dbg = g_gru_dbg;
-  p.ablate = g_gru_ablate & 31;
   p.ring = ring; p.gc = gc;
   CUtensorMap tm[2];
   for (int d = 0; d < 2; ++d) {
@@ -2082,8 +1989,7 @@ extern "C" int sb_gru_fwd(const float* gi, const void* whh_bf16, const float* bh
     if (rc != SB_OK) return rc;
   }
   void* args[] = {(void*)&tm[0], (void*)&tm[1], (void*)&p};
-  return gru_launch((const void*)gru_fwd_kernel, ndir * nC, gru_cluster_size(nC), smem, args,
-                    stream);
+  return gru_launch((const void*)gru_fwd_kernel, ndir * nC, nC, 4, 1, smem, args, stream);
 }
 
 extern "C" int sb_gru_bwd_workspace_size(int Bp, int H, int ndir, size_t* bytes) {
@@ -2091,7 +1997,7 @@ extern "C" int sb_gru_bwd_workspace_size(int Bp, int H, int ndir, size_t* bytes)
   // counters + the double-buffered exchange of dgh_t (Bp x 3H bf16 per direction and parity; the
   // tile-major form of the K-split kernel rounds 3H up to whole 64-column chunks)
   const size_t k3p = (size_t)((3 * H + 63) / 64) * 64;
-  *bytes = gru_ws_counters_bytes(ndir) + (size_t)ndir * 2 * Bp * k3p * sizeof(bf16) + 1024;
+  *bytes = GRU_WS_COUNTERS + (size_t)ndir * 2 * Bp * k3p * sizeof(bf16) + 1024;
   return SB_OK;
 }
 
@@ -2115,10 +2021,9 @@ extern "C" int sb_gru_bwd(const float* dy, const float* y, const float* gates,
   p.dgi = reinterpret_cast<bf16*>(dgi_bf16);
   p.dghn = reinterpret_cast<bf16*>(dghn_bf16);
   p.barrier = reinterpret_cast<unsigned int*>(ws);
-  p.xchg = reinterpret_cast<bf16*>(ws + gru_ws_counters_bytes(ndir));
+  p.xchg = reinterpret_cast<bf16*>(ws + GRU_WS_COUNTERS);
   p.dbih = dbih; p.dbhh = dbhh; p.T = T; p.Bp = Bp; p.H = H; p.ndir = ndir;
   p.dbg = g_gru_dbg;
-  p.ablate = g_gru_ablate & 192;
   const int K3 = 3 * H;
   const int nchunks = (K3 + 63) / 64;
   size_t smem = 0;
@@ -2127,7 +2032,7 @@ extern "C" int sb_gru_bwd(const float* dy, const float* y, const float* gates,
   // partial chunk are never written and must read as zero)
   if (cudaMemsetAsync(workspace, 0, need, stream) != cudaSuccess) return SB_ERR_CUDA;
   // ---- preferred: K-split over 4-CTA clusters ----
-  if (g_gru_ksplit && H % 256 == 0 && nC_ % KS == 0 && (K3 / KS / 64) <= 16) {
+  if (H % 256 == 0 && nC_ % KS == 0 && (K3 / KS / 64) <= 16) {
     const int nq = K3 / KS / 64;
     const size_t ks_smem = (size_t)nq * Bp * 128 + (size_t)nq * 64 * 128 +
                            (size_t)2 * KS * Bp * 64 + 1024 + 256;
@@ -2144,13 +2049,12 @@ extern "C" int sb_gru_bwd(const float* dy, const float* y, const float* gates,
       const size_t kt_smem = (size_t)nq * Bp * 128 + (size_t)nq * 64 * 128 +
                              std::max(ex, (size_t)8192) + 1024 + 256;
       if (gru_use_kt(Bp, true) && kt_smem <= 227 * 1024) {
-        const void* kt = Bp > 32   ? (const void*)gru_bwd_kt_kernel<4>
-                         : Bp > 16 ? (const void*)gru_bwd_kt_kernel<2>
-                                   : (const void*)gru_bwd_kt_kernel<1>;
-        rc = gru_launch_exact(kt, ndir * nC_, KS, kt_smem, kargs, stream);
+        rc = gru_launch((const void*)gru_bwd_kt_kernel<1>, ndir * nC_, nC_, KS, KS, kt_smem, kargs,
+                        stream);
         if (rc == SB_OK) return SB_OK;
       }
-      rc = gru_launch_exact((const void*)gru_bwd_ks_kernel, ndir * nC_, KS, ks_smem, kargs, stream);
+      rc = gru_launch((const void*)gru_bwd_ks_kernel, ndir * nC_, nC_, KS, KS, ks_smem, kargs,
+                      stream);
       if (rc == SB_OK) return SB_OK;
     }
   }
@@ -2164,7 +2068,5 @@ extern "C" int sb_gru_bwd(const float* dy, const float* y, const float* gates,
     if (rc != SB_OK) return rc;
   }
   void* args[] = {(void*)&tm[0], (void*)&tm[1], (void*)&p};
-  const int nC = H / GRU_HC;
-  return gru_launch((const void*)gru_bwd_kernel, ndir * nC, gru_cluster_size(nC), smem, args,
-                    stream);
+  return gru_launch((const void*)gru_bwd_kernel, ndir * nC_, nC_, 4, 1, smem, args, stream);
 }

@@ -20,23 +20,6 @@ def _round_up(x, m):
     return (x + m - 1) // m * m
 
 
-def _apply_env_knobs():
-    """Developer knobs (profiling under ncu cannot replay clustered cooperative launches):
-    SB_GRU_KSPLIT=0 disables the K-split backward kernel, SB_GRU_CLUSTER=<1|2|4|8> sets the
-    preferred cluster size of the other GRU kernels."""
-    import os
-    lib = _lib.load()
-    if os.environ.get("SB_GRU_KSPLIT") is not None:
-        lib.sb_debug_gru_ksplit(int(os.environ["SB_GRU_KSPLIT"]))
-    if os.environ.get("SB_GEMM_MT1") is not None:
-        lib.sb_debug_gemm_mt1(int(os.environ["SB_GEMM_MT1"]))
-    if os.environ.get("SB_GRU_CLUSTER") is not None:
-        lib.sb_debug_gru_cluster(int(os.environ["SB_GRU_CLUSTER"]))
-
-
-_knobs_applied = False
-
-
 # ---- optional per-kernel timing (CUDA events on the launching stream; used by bench.py) ----
 _prof = None
 _prof_detail = False      # developer: one profile class per GEMM shape (tools/debug_step.py)
@@ -61,10 +44,6 @@ def profile_end():
 
 def _launch(name, flops, fn):
     """Run one C-ABI launch; counts it and, when profiling, brackets it with CUDA events."""
-    global _knobs_applied
-    if not _knobs_applied:
-        _knobs_applied = True
-        _apply_env_knobs()
     _lib.launch_count += 1
     if _prof is None:
         return _lib.check(fn(), name)
@@ -595,25 +574,6 @@ def gru_stack(x, rnn, dropout=0.0):
         xc, ndir, rnn.hidden_size, float(dropout), None, None, *weights))
 
 
-def _transpose_bf16(src, rows_pad=8, out=None):
-    """[R][C] bf16 -> [C][Rp] bf16 (Rp = R rounded up so that rows stay 16-byte aligned);
-    `out` (optional): a [C][>=R] bf16 destination with contiguous rows."""
-    lib = _lib.load()
-    R, C = src.shape
-    Rp = _round_up(R, rows_pad)
-    if out is not None:
-        dst = out
-    elif Rp != R:
-        dst = torch.zeros(C, Rp, dtype=torch.bfloat16, device=src.device)
-    else:
-        dst = torch.empty(C, Rp, dtype=torch.bfloat16, device=src.device)
-    sp = _lib.stream_ptr()
-    _launch("transpose_bf16", 0.0,
-            lambda: lib.sb_transpose_bf16(src.data_ptr(), dst.data_ptr(), R, C, src.stride(0),
-                                          dst.stride(0), sp))
-    return dst[:, :R]
-
-
 class ConvStackFunction(torch.autograd.Function):
     """Conv2d+ReLU stack as im2col + tcgen05 GEMM (csrc/conv.cu, csrc/gemm.cu).
 
@@ -723,12 +683,7 @@ def conv_stack(x, conv, training):
 
     x (B, T, F) -> (B, T', C*F') with the reference's channel-major feature flattening
     (transpose(1,2) of (B,C,T',F') then view, model.py:66-71).  Runs on our im2col + tcgen05
-    kernels, including the Dropout after each ReLU when training.  Shapes the kernels do not
-    cover go through the nn modules: grouped / dilated / padded convolutions and out_channels not
-    a multiple of 8 (none of which the reference can express, model.py:21-23), and - only when a
-    gradient is needed - an upper layer whose kernel spans more than 5 x 8 taps per stride phase
-    (the unrolled gather of `col2im_relu_kernel`; the TIMIT recipes' second layer [*, 5, 32, 1]
-    is the one shipped case: its forward / inference still runs on our kernels).
+    kernels, including the Dropout after each ReLU when training.
     """
     mods = list(conv.children())
     convs = [m for m in mods if isinstance(m, torch.nn.Conv2d)]

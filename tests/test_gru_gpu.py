@@ -80,17 +80,13 @@ def test_gru_large_per_gpu_batch(cuda_lib, B, H):
         assert (pc.grad.double().cpu() - ref).abs().max().item() < 3e-2 * ref.abs().max().item() + 1e-4, n
 
 
-@pytest.mark.parametrize("flavour", [8, 16])
 @pytest.mark.parametrize("B", [8, 20, 33, 56, 64])
-def test_gru_both_k_split_flavours(cuda_lib, B, flavour):
+def test_gru_both_k_split_flavours(cuda_lib, B):
     """The two K-split recurrence kernels (batch-major accumulator `ks`, transposed accumulator
-    `kt`; csrc/gru.cu picks by batch size) forced in turn through the developer knob, forward and
-    backward, at padded batch sizes 8/24/40/56/64 that exercise every units-per-thread variant."""
-    cuda_lib.sb_debug_gru_flags(flavour)       # 8: ks only, 16: kt always
-    try:
-        rnn64, x64, y64, rnn_c, xc, yc = _ref_and_ours(B, 7, 96, 256, 2, True, seed=B + flavour)
-    finally:
-        cuda_lib.sb_debug_gru_flags(0)
+    `kt`), forward and backward.  csrc/gru.cu picks the flavour by padded batch size; 8/24/40/56/64
+    rows reach every kernel the selection can pick: forward `kt<1>` at 8, `kt<2>` at 24, `ks` at
+    40-64; backward `kt<1>` at 8, `ks` at 24-64."""
+    rnn64, x64, y64, rnn_c, xc, yc = _ref_and_ours(B, 7, 96, 256, 2, True, seed=B)
     assert (yc.double().cpu() - y64).abs().max().item() < 2e-2
     gx = xc.grad.double().cpu()
     assert (gx - x64.grad).abs().max().item() < 3e-2 * x64.grad.abs().max().item() + 1e-4

@@ -1,22 +1,19 @@
-"""Developer tool: per-step timeline (ns) of CTA 0 of the GRU forward kernel at north-star width."""
+"""Developer tool: per-step timeline (ns) of CTA 0 of the GRU recurrence at north-star width.
+
+    python tools/gru_timeline.py [fwd|bwd]      (TL_B=<batch>, default 64)
+"""
 import sys
 import numpy as np, torch
 sys.path.insert(0, ".")
 from speech_b200 import _lib, ops
 lib = _lib.load()
-if len(sys.argv) > 1:
-    lib.sb_debug_gru_cluster(int(sys.argv[1]))
-    print("cluster size preference:", sys.argv[1])
-if len(sys.argv) > 3:
-    lib.sb_debug_gru_flags(int(sys.argv[3]))      # 32: version-1 forward kernel
-    print("flags:", sys.argv[3])
 torch.manual_seed(0)
 import os
 B, T, In, H = int(os.environ.get('TL_B', '64')), 64, 2048, 1024
 rnn = torch.nn.GRU(In, H, 1, batch_first=True, bidirectional=True).cuda()
 x = torch.randn(B, T, In, device="cuda")
 dbg = torch.zeros(64 * 16 + 512, dtype=torch.int64, device="cuda")
-MODE = sys.argv[2] if len(sys.argv) > 2 else "fwd"
+MODE = sys.argv[1] if len(sys.argv) > 1 else "fwd"
 if MODE == "fwd":
     with torch.no_grad():
         ops.gru_stack(x, rnn)
