@@ -278,11 +278,4 @@ SB_DEVINL uint32_t pack_bf16x2(float lo, float hi) {
   return *reinterpret_cast<uint32_t*>(&t);
 }
 
-SB_DEVINL float sigmoidf_fast(float x) { return 1.0f / (1.0f + __expf(-x)); }
-SB_DEVINL float tanhf_fast(float x) {
-  // tanh(x) = 1 - 2/(exp(2x)+1); exact limits at +-inf, abs err ~1e-7 near 0
-  float e = __expf(2.0f * x);
-  return 1.0f - 2.0f / (e + 1.0f);
-}
-
 }  // namespace sb

@@ -7,23 +7,23 @@
 //
 // The time-batched input projection gi = X W_ih^T + b_ih is done for all T at once by
 // sb_gemm_bf16_tn; these kernels run the T-serial part.  One launch per layer covers BOTH
-// directions:
-//   * CTA c of direction d owns 16 hidden units j0..j0+15: its 48 rows of W_hh (r,z,n) stay
-//     resident in shared memory (bf16, UMMA K-major SWIZZLE_128B chunks) for all T steps;
-//   * per step every CTA needs ALL of h_{t-1} (bf16, written by the CTAs of its direction in the
-//     previous step).  CTAs form thread-block clusters of up to 4; each CTA fetches 1/CS of the
-//     [Bp x 64] chunks with TMA and MULTICASTS them into the shared memory of all CTAs of its
-//     cluster, so L2 is read once per cluster instead of once per CTA (the un-multicast version
-//     was bound by 64 SMs hammering the same L2 lines: 4 us of a 13 us step);
-//   * one thread issues tcgen05.mma  D[batch(128) x 48] += h_{t-1}[batch x 64] * Wslice[48 x 64]^T
-//     per chunk as its mbarrier completes; accumulators live in TMEM;
-//   * 8 epilogue warps (thread = TMEM lane = batch row, 8 hidden units each) read the
-//     accumulators with tcgen05.ld, apply the gate math in fp32 (h_{t-1} of the thread's own units
-//     stays in registers across steps), publish the bf16 h_t, arrive on the per-direction grid
-//     barrier, and only then write the fp32 state / saved gates;
-//   * the grid barrier is one red.release.gpu + ld.acquire.gpu polling on a global counter.
-// The backward kernel has the same structure with W_hh^T resident (16 rows x 3H) and the
-// all-gather over the pre-activation gradients dgh_t (batch x 3H).
+// directions.  CTA c of direction d does the gate math of 16 hidden units, and the CTAs of a
+// direction meet once per step at a grid barrier (one red.release.gpu + ld.acquire.gpu polling on a
+// global counter).  Six kernels, three per direction of time:
+//   * gru_fwd_kernel / gru_bwd_kernel (full gather): every CTA gathers ALL of h_{t-1} (backward:
+//     the pre-activation gradients dgh_t, batch x 3H) through a ring of shared-memory slots, with
+//     TMA multicast inside clusters of up to 4.  Any H % 16 == 0, up to 128 batch rows.
+//   * gru_fwd_ks_kernel / gru_bwd_ks_kernel (K split): the 4 CTAs of a cluster jointly own 64
+//     units; CTA r contracts only the r-th quarter of K into a batch-major accumulator, and the
+//     partial products are reduce-scattered through distributed shared memory.  H % 256 == 0.
+//   * gru_fwd_kt_kernel<UPT> / gru_bwd_kt_kernel (K split, transposed accumulator): the same
+//     partition with the weights as the M-side operand, for small batches.
+// All six have the same warp roles (warps 0..7 epilogue: TMEM -> gate math -> publish -> off-path
+// stores; warp 8 MMA issuer and TMEM owner; warp 9 TMA producer) and share what is written once
+// below: the shared-memory layout of each family (GruSmemLayout, which the kernels carve and the
+// host sizes the launch from), setup and teardown, the per-thread loads and stores of UPT units,
+// the gate math of each direction with its publish and off-path stores, and the K-split gather
+// and MMA of each direction.  What differs is the exchange and the accumulator layout.
 //
 // Roofline: tensor work, but each step is bound by the all-gather + barrier latency; DESIGN.md
 // reports us/step next to the tensor-pipe share.
@@ -37,10 +37,12 @@
 namespace sb {
 
 static constexpr int GRU_HC = 16;            // hidden units per CTA
-static constexpr int GRU_UPT = 8;            // hidden units per epilogue thread
+static constexpr int GRU_UPT = 8;            // hidden units per epilogue thread (batch-major)
 static constexpr int GRU_MAX_RING = 16;      // smem ring slots for the gathered operand
 static constexpr int GRU_EPI = 256;          // warps 0..7: epilogue
 static constexpr int GRU_THREADS = GRU_EPI + 64;  // + warp 8: MMA issuer/TMEM owner, warp 9: TMA
+static constexpr int KS = 4;                 // K split: CTAs of a cluster, quarters of K
+static constexpr int GRU_KS_BWD_GROUPS = 4;  // K split, backward: full barriers (chunk groups)
 
 typedef __nv_bfloat16 bf16;
 
@@ -70,6 +72,133 @@ struct GruBwdParams {
   unsigned long long* dbg;
   int T, Bp, H, ndir, ring, gc;
 };
+
+// =============================================================================================
+// shared-memory layout
+// =============================================================================================
+// One layout per kernel family.  The kernel carves its shared memory from it and the host requests
+// `bytes` and decides from it whether the kernel fits, so the two cannot disagree.  Offsets are in
+// bytes from the 1024-aligned base of dynamic shared memory; the gather ring starts at 0, and
+// everything below `full` is zeroed at setup.
+struct GruSmemLayout {
+  int wtile;      // resident weight chunks (wrows x 64 bf16 each, K-major SWIZZLE_128B)
+  int recv;       // K split: partial products received from the peers
+  int stage;      // K split: partial products staged for the peers
+  int full;       // `nfull` mbarriers: gathered chunks landed
+  int nfull;
+  int empty;      // full gather: GRU_MAX_RING mbarriers, ring slot free (0 = none)
+  int accfull;    // mbarrier: accumulator complete
+  int recvbar;    // K split: mbarrier, the peers' slices landed (0 = none)
+  int tmem_slot;  // TMEM base address written by tcgen05.alloc
+  int scratch;    // b_hh of the CTA's units (forward); bias-gradient reduction (full-gather bwd)
+  int bytes;      // dynamic shared memory to request (alignment slack and reserved tail included)
+};
+
+__host__ __device__ __forceinline__ int gru_imax(int a, int b) { return a > b ? a : b; }
+
+// Chunks of the gathered operand share one mbarrier per group of gc: the largest of 4, 3, 2, 1
+// that divides nchunks.
+__host__ __device__ __forceinline__ int gru_group_chunks(int nchunks) {
+  return nchunks % 4 == 0 ? 4 : (nchunks % 3 == 0 ? 3 : (nchunks % 2 == 0 ? 2 : 1));
+}
+
+// Full gather: ring | weights | barriers | scratch.  The 128-row MMA read of the last ring slot
+// overruns by (16 KB - Bp*128) into the weight region, which is padded to cover it.
+__host__ __device__ __forceinline__ GruSmemLayout gru_layout_full(int Bp, int nchunks, int wrows,
+                                                                 int ring_bytes) {
+  GruSmemLayout L;
+  L.wtile = ring_bytes;
+  L.full = L.wtile + gru_imax(nchunks * wrows * 128, 16384 - Bp * 128);
+  L.recv = L.stage = L.full;
+  L.nfull = GRU_MAX_RING;
+  L.empty = L.full + GRU_MAX_RING * 8;
+  L.accfull = L.empty + GRU_MAX_RING * 8;
+  L.recvbar = 0;
+  L.tmem_slot = L.accfull + 8;
+  L.scratch = L.tmem_slot + 8;
+  L.bytes = 1024 + L.scratch + 64 * 4 + 64;
+  return L;
+}
+
+// K split: the whole K quarter is resident (ring of nchunks slots) | weights | receive and staging
+// buffers of the reduce-scatter (at least xchg_min bytes together) | barriers | `tail` bytes for
+// the TMEM slot and the bias.
+__host__ __device__ __forceinline__ GruSmemLayout gru_layout_ksplit(int Bp, int nchunks, int wrows,
+                                                                   int recv_bytes, int stage_bytes,
+                                                                   int xchg_min, int nfull,
+                                                                   int tail) {
+  GruSmemLayout L;
+  L.wtile = nchunks * Bp * 128;
+  L.recv = L.wtile + nchunks * wrows * 128;
+  L.stage = L.recv + recv_bytes;
+  L.full = L.recv + gru_imax(recv_bytes + stage_bytes, xchg_min);
+  L.nfull = nfull;
+  L.empty = 0;
+  L.accfull = L.full + nfull * 8;
+  L.recvbar = L.accfull + 8;
+  L.tmem_slot = L.recvbar + 8;
+  L.scratch = L.tmem_slot + 8;
+  L.bytes = 1024 + L.full + tail;
+  return L;
+}
+
+// ks forward: 192 weight rows (gate x 64 units); [KS][Bp][48] floats received and staged.  The
+// 128-row A read of the last chunk runs past the ring into the weights (finite, rows >= Bp unused).
+__host__ __device__ __forceinline__ GruSmemLayout gru_layout_fwd_ks(int Bp, int H) {
+  const int xb = KS * Bp * 3 * GRU_HC * 4;
+  return gru_layout_ksplit(Bp, H / KS / 64, 3 * KS * GRU_HC, xb, xb, 0, 1, 512);
+}
+// ks backward: 64 weight rows (units of W_hh^T); [KS][Bp][16] floats received and staged.
+__host__ __device__ __forceinline__ GruSmemLayout gru_layout_bwd_ks(int Bp, int H) {
+  const int xb = KS * Bp * GRU_HC * 4;
+  return gru_layout_ksplit(Bp, 3 * H / KS / 64, KS * GRU_HC, xb, xb, 0, GRU_KS_BWD_GROUPS, 256);
+}
+// kt forward: slices of [48][Bp+4] floats, KS received and KS-1 staged.  The N-side read of the
+// last chunk runs up to 8 rows past the ring into the weights, and the 128-row M-side read of tile
+// 1 runs 64 rows past its 64 valid ones (into the next chunk / the receive buffer): both only feed
+// accumulator columns / lanes that are never read.
+__host__ __device__ __forceinline__ GruSmemLayout gru_layout_fwd_kt(int Bp, int H) {
+  const int slice = 3 * GRU_HC * (Bp + 4) * 4;
+  return gru_layout_ksplit(Bp, H / KS / 64, 3 * KS * GRU_HC, KS * slice, (KS - 1) * slice, 0, 1,
+                           512);
+}
+// kt backward: slices of [16][Bp+4] floats.  The 128-row M-side read of the last weight chunk
+// needs 8 KB after the weights, which the exchange buffers cover only for large batches.
+__host__ __device__ __forceinline__ GruSmemLayout gru_layout_bwd_kt(int Bp, int H) {
+  const int slice = GRU_HC * (Bp + 4) * 4;
+  return gru_layout_ksplit(Bp, 3 * H / KS / 64, KS * GRU_HC, KS * slice, (KS - 1) * slice, 8192,
+                           GRU_KS_BWD_GROUPS, 256);
+}
+
+struct GruSmem {
+  uint8_t* ring;
+  uint8_t* wtile;
+  float* recv;
+  float* stage;
+  uint64_t* full;
+  uint64_t* empty;
+  uint64_t* accfull;
+  uint64_t* recvbar;
+  uint32_t* tmem_slot;
+  float* scratch;
+};
+
+SB_DEVINL GruSmem gru_carve(uint8_t* raw, const GruSmemLayout& L) {
+  uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(raw) + 1023) &
+                                             ~static_cast<uintptr_t>(1023));
+  GruSmem s;
+  s.ring = base;
+  s.wtile = base + L.wtile;
+  s.recv = reinterpret_cast<float*>(base + L.recv);
+  s.stage = reinterpret_cast<float*>(base + L.stage);
+  s.full = reinterpret_cast<uint64_t*>(base + L.full);
+  s.empty = reinterpret_cast<uint64_t*>(base + L.empty);
+  s.accfull = reinterpret_cast<uint64_t*>(base + L.accfull);
+  s.recvbar = reinterpret_cast<uint64_t*>(base + L.recvbar);
+  s.tmem_slot = reinterpret_cast<uint32_t*>(base + L.tmem_slot);
+  s.scratch = reinterpret_cast<float*>(base + L.scratch);
+  return s;
+}
 
 SB_DEVINL unsigned long long gtime() {
   unsigned long long t;
@@ -127,32 +256,69 @@ SB_DEVINL void umma_commit_mc(uint64_t* bar, uint16_t mask) {
       " [%0], %1;" ::"r"(smem_u32(bar)), "h"(mask)
       : "memory");
 }
-
-struct GruSmem {
-  uint8_t* ring;    // ring slots (stride = Bp*128 bytes), placed BEFORE the weights so that the
-                    // 128-row MMA read of the last slot overruns into (finite) weight data
-  uint8_t* wtile;   // resident weight chunks
-  uint64_t* full;   // [GRU_MAX_RING]
-  uint64_t* empty;  // [GRU_MAX_RING]
-  uint64_t* accfull;
-  uint32_t* tmem_slot;
-  float* scratch;   // [64]
-};
-
-SB_DEVINL GruSmem carve(uint8_t* raw, int ring_bytes, int wbytes) {
-  GruSmem s;
-  s.ring = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(raw) + 1023) &
-                                      ~static_cast<uintptr_t>(1023));
-  s.wtile = s.ring + ring_bytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(s.wtile + wbytes);
-  s.full = bars;
-  s.empty = bars + GRU_MAX_RING;
-  s.accfull = bars + 2 * GRU_MAX_RING;
-  s.tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * GRU_MAX_RING + 1);
-  s.scratch = reinterpret_cast<float*>(bars + 2 * GRU_MAX_RING + 2);
-  return s;
+SB_DEVINL uint32_t mapa_shared(uint32_t local_addr, uint32_t peer) {
+  uint32_t r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_addr), "r"(peer));
+  return r;
+}
+// bulk copy from this CTA's shared memory into a PEER's shared memory (DSMEM through the copy
+// engine), completing `bytes` on the peer's mbarrier.  Measured: pushing the reduce-scatter
+// slices with per-thread st.shared::cluster took 4.1 us for 36 KB (~9 KB/us per SM).
+SB_DEVINL void bulk_s2peer(uint32_t peer_dst, const void* local_src, uint32_t bytes,
+                           uint32_t peer_bar) {
+  asm volatile(
+      "cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+      ::"r"(peer_dst), "r"(smem_u32(local_src)), "r"(bytes), "r"(peer_bar)
+      : "memory");
 }
 
+// ---- setup and teardown -----------------------------------------------------------------------
+// Zero the ring, weight and exchange regions (rows past the batch and columns past K must read as
+// finite zeros), stage the resident operand (`stage`, which differs per kernel), initialise the
+// barriers, allocate `tmem_cols` TMEM columns, and make all of it visible to the async proxy and to
+// the peer CTAs before any of them multicasts or copies into this CTA.  The empty barriers of the
+// full gather count one arrive per CTA of the cluster (`cluster_ctas`).  Returns the TMEM base.
+template <class Stage>
+SB_DEVINL uint32_t gru_setup(const GruSmem& s, const GruSmemLayout& L, const CUtensorMap* tm,
+                             uint32_t tmem_cols, uint32_t cluster_ctas, Stage stage) {
+  const int tid = threadIdx.x;
+  for (int k = tid; k < L.full / 16; k += GRU_THREADS)
+    reinterpret_cast<uint4*>(s.ring)[k] = make_uint4(0, 0, 0, 0);
+  __syncthreads();
+  stage();
+  if (tid == 0) {
+    for (int i = 0; i < L.nfull; ++i) {
+      mbar_init(&s.full[i], 1);
+      if (L.empty) mbar_init(&s.empty[i], cluster_ctas);
+    }
+    mbar_init(s.accfull, 1);
+    // one local arrive.expect_tx per step; the peers' copies complete_tx
+    if (L.recvbar) mbar_init(s.recvbar, 1);
+    mbar_fence_init();
+    tma_prefetch_desc(tm);
+  }
+  if ((tid >> 5) == 8) tmem_alloc(s.tmem_slot, tmem_cols);
+  fence_proxy_async_smem();
+  tc_fence_before_sync();
+  __syncthreads();
+  tc_fence_after_sync();
+  cluster_sync_all();   // peers' barriers are initialised before anyone multicasts into them
+  return *s.tmem_slot;
+}
+
+SB_DEVINL void gru_teardown(uint32_t tmem_base, uint32_t tmem_cols) {
+  tc_fence_before_sync();
+  __syncthreads();
+  cluster_sync_all();   // no CTA leaves while peers may still signal its barriers
+  if ((threadIdx.x >> 5) == 8) {
+    tc_fence_after_sync();
+    tmem_dealloc(tmem_base, tmem_cols);
+  }
+}
+
+// =============================================================================================
+// full gather: ring of gathered chunks
+// =============================================================================================
 // The gathered operand of one step is `nchunks` [Bp x 64] boxes, handled in groups of `gc` chunks
 // that share ONE full/empty mbarrier pair (an mbarrier wait costs ~100 ns even when it is already
 // complete, so per-chunk barriers were 3 us of a 10 us step).  Group g uses ring slot g % ring and
@@ -213,6 +379,102 @@ SB_DEVINL void mma_consume(const GruSmem& s, uint32_t tmem_d, int nchunks, int w
   umma_commit(s.accfull);
 }
 
+// =============================================================================================
+// K split: one step of the gather and of the product, per direction
+// =============================================================================================
+// Forward: the CTA's K quarter of h_{t-1} (columns col0.., rows row0.. of xn) stays resident
+// whole, behind ONE full barrier.
+SB_DEVINL void ks_gather_fwd(const GruSmem& s, const CUtensorMap* tm, int stride, int nchunks,
+                             int col0, int row0) {
+  mbar_expect_tx(s.full, (uint32_t)(stride * nchunks));
+  for (int c = 0; c < nchunks; ++c)
+    tma_load_2d(s.ring + c * stride, tm, s.full, col0 + c * 64, row0);
+}
+// Batch-major (ks): D[batch x 192] = h * W^T.  Transposed (kt): D0[128 x NB] = W(r,z rows) * h^T
+// at TMEM column 0 and D1 = W(n rows) * h^T at column 64, the weight chunk being the M-side
+// operand and `idesc` of N = NB.
+SB_DEVINL void ks_mma_fwd(const GruSmem& s, uint32_t tmem, int stride, int nchunks, int wchunk,
+                          uint32_t idesc, bool transposed, uint32_t parity) {
+  mbar_wait(s.full, parity);
+  tc_fence_after_sync();
+  for (int c = 0; c < nchunks; ++c) {
+    const uint64_t dh = umma_desc_sw128_kmajor(smem_u32(s.ring + c * stride));
+    const uint64_t dw = umma_desc_sw128_kmajor(smem_u32(s.wtile + c * wchunk));
+    if (!transposed) {
+#pragma unroll
+      for (int kk = 0; kk < 4; ++kk)
+        umma_bf16_ss(tmem, dh + (uint64_t)(kk * 2), dw + (uint64_t)(kk * 2), idesc,
+                     (c > 0 || kk > 0) ? 1u : 0u);
+    } else {
+      const uint64_t dw1 = umma_desc_sw128_kmajor(smem_u32(s.wtile + c * wchunk + 128 * 128));
+#pragma unroll
+      for (int kk = 0; kk < 4; ++kk) {
+        const uint32_t acc = (c > 0 || kk > 0) ? 1u : 0u;
+        umma_bf16_ss(tmem, dw + (uint64_t)(kk * 2), dh + (uint64_t)(kk * 2), idesc, acc);
+        umma_bf16_ss(tmem + 64, dw1 + (uint64_t)(kk * 2), dh + (uint64_t)(kk * 2), idesc, acc);
+      }
+    }
+  }
+  umma_commit(s.accfull);
+}
+
+// Backward: the CTA's K quarter of dgh_t (3H/4 columns) in groups of gc chunks, one full barrier
+// per group (at most GRU_KS_BWD_GROUPS groups; the host checks).
+SB_DEVINL void ks_gather_bwd(const GruSmem& s, const CUtensorMap* tm, int stride, int ngroups,
+                             int gc, int col0, int row0) {
+  for (int g = 0; g < ngroups; ++g) {
+    mbar_expect_tx(&s.full[g], (uint32_t)(stride * gc));
+    for (int i = 0; i < gc; ++i) {
+      const int c = g * gc + i;
+      tma_load_2d(s.ring + c * stride, tm, &s.full[g], col0 + c * 64, row0);
+    }
+  }
+}
+// Batch-major (ks): D[batch x 64 units] = dgh * W_hh.  Transposed (kt): D^T[64 units x NB], the
+// weight chunk being the M-side operand.
+SB_DEVINL void ks_mma_bwd(const GruSmem& s, uint32_t tmem, int stride, int ngroups, int gc,
+                          int wchunk, uint32_t idesc, bool transposed, uint32_t parity) {
+  for (int g = 0; g < ngroups; ++g) {
+    mbar_wait(&s.full[g], parity);
+    tc_fence_after_sync();
+    for (int i = 0; i < gc; ++i) {
+      const int c = g * gc + i;
+      const uint64_t dh = umma_desc_sw128_kmajor(smem_u32(s.ring + c * stride));
+      const uint64_t dw = umma_desc_sw128_kmajor(smem_u32(s.wtile + c * wchunk));
+      const uint64_t da = transposed ? dw : dh, db = transposed ? dh : dw;
+#pragma unroll
+      for (int kk = 0; kk < 4; ++kk)
+        umma_bf16_ss(tmem, da + (uint64_t)(kk * 2), db + (uint64_t)(kk * 2), idesc,
+                     (c > 0 || kk > 0) ? 1u : 0u);
+    }
+  }
+  umma_commit(s.accfull);
+}
+
+// Backward staging of the K-split kernels: rows = the cluster's 64 units of W_hh^T (k0c..),
+// columns = the CTA's K quarter.  W_hh is read as stored ([3H][H]: the cluster's 64 units are 128
+// contiguous bytes of row k) and transposed on the way into shared memory.  The 64 rows are grouped
+// by owner: rows 16q..16q+15 belong to CTA q of the cluster.
+SB_DEVINL void ks_stage_whh_t(uint8_t* wtile, const bf16* whh, int H, int dir, int k0c,
+                              uint32_t crank) {
+  constexpr int WCHUNK = 64 * 128;
+  const int K3 = 3 * H, KQ = K3 / KS;
+  for (int k = threadIdx.x; k < KQ * 8; k += GRU_THREADS) {
+    const int kl = k >> 3, piece = k & 7;       // local k, 8-unit piece of the 64 units
+    const uint4 v = *reinterpret_cast<const uint4*>(
+        whh + ((long long)dir * K3 + (long long)crank * KQ + kl) * H + k0c + piece * 8);
+    const unsigned short* e = reinterpret_cast<const unsigned short*>(&v);
+    uint8_t* chunk = wtile + (kl >> 6) * WCHUNK + (kl & 7) * 2;
+#pragma unroll
+    for (int q = 0; q < 8; ++q)
+      *reinterpret_cast<unsigned short*>(
+          chunk + sw128_offset((uint32_t)(piece * 8 + q), (uint32_t)((kl & 63) >> 3))) = e[q];
+  }
+}
+
+// =============================================================================================
+// per-thread work: UPT consecutive units of one batch row (8 batch-major, 1 or 2 in kt)
+// =============================================================================================
 SB_DEVINL float fast_sigmoid(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
 SB_DEVINL float fast_tanh(float x) {
   // 1 - 2/(exp(2x)+1), clamped so exp never overflows (__fdividef(2, inf) is not guaranteed 0)
@@ -220,29 +482,62 @@ SB_DEVINL float fast_tanh(float x) {
   return 1.0f - __fdividef(2.0f, __expf(2.0f * xc) + 1.0f);
 }
 
-// One-touch data (gi, saved gates, dy, fp32 state, GEMM operands written for later kernels) uses
-// the streaming cache policy (.cs) so that it does not evict the latency-critical bf16 exchange
-// buffers, which every CTA re-reads from L2 each step.
-SB_DEVINL void ld8(const float* p, float (&v)[8]) {
-  const float4 a = __ldcs(reinterpret_cast<const float4*>(p));
-  const float4 b = __ldcs(reinterpret_cast<const float4*>(p) + 1);
-  v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
-}
-SB_DEVINL void st8(float* p, const float (&v)[8]) {
-  __stcs(reinterpret_cast<float4*>(p), make_float4(v[0], v[1], v[2], v[3]));
-  __stcs(reinterpret_cast<float4*>(p) + 1, make_float4(v[4], v[5], v[6], v[7]));
-}
-SB_DEVINL void st_stream_u4(void* p, uint4 v) { __stcs(reinterpret_cast<uint4*>(p), v); }
-SB_DEVINL void st_stream_bf16(bf16* p, float v) {
-  const unsigned short u = __bfloat16_as_ushort(__float2bfloat16_rn(v));
-  asm volatile("st.global.cs.u16 [%0], %1;" ::"l"(p), "h"(u) : "memory");
-}
 SB_DEVINL uint4 pack8(const float (&v)[8]) {
   uint4 r;
   r.x = pack_bf16x2(v[0], v[1]); r.y = pack_bf16x2(v[2], v[3]);
   r.z = pack_bf16x2(v[4], v[5]); r.w = pack_bf16x2(v[6], v[7]);
   return r;
 }
+// One-touch data (gi, saved gates, dy, fp32 state, GEMM operands written for later kernels) uses
+// the streaming cache policy (.cs) so that it does not evict the latency-critical bf16 exchange
+// buffers, which every CTA re-reads from L2 each step.
+template <int UPT>
+SB_DEVINL void ldu(const float* p, float (&v)[UPT]) {
+  if constexpr (UPT == 8) {
+    const float4 a = __ldcs(reinterpret_cast<const float4*>(p));
+    const float4 b = __ldcs(reinterpret_cast<const float4*>(p) + 1);
+    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+  } else if constexpr (UPT == 2) {
+    const float2 a = __ldcs(reinterpret_cast<const float2*>(p));
+    v[0] = a.x; v[1] = a.y;
+  } else {
+    v[0] = __ldcs(p);
+  }
+}
+template <int UPT>
+SB_DEVINL void stu(float* p, const float (&v)[UPT]) {
+  if constexpr (UPT == 8) {
+    __stcs(reinterpret_cast<float4*>(p), make_float4(v[0], v[1], v[2], v[3]));
+    __stcs(reinterpret_cast<float4*>(p) + 1, make_float4(v[4], v[5], v[6], v[7]));
+  } else if constexpr (UPT == 2) {
+    __stcs(reinterpret_cast<float2*>(p), make_float2(v[0], v[1]));
+  } else {
+    __stcs(p, v[0]);
+  }
+}
+// the bf16 exchange, re-read by every CTA: default cache policy
+template <int UPT>
+SB_DEVINL void st_bf16u(bf16* p, const float (&v)[UPT]) {
+  if constexpr (UPT == 8) {
+    *reinterpret_cast<uint4*>(p) = pack8(v);
+  } else if constexpr (UPT == 2) {
+    *reinterpret_cast<uint32_t*>(p) = pack_bf16x2(v[0], v[1]);
+  } else {
+    *p = __float2bfloat16_rn(v[0]);
+  }
+}
+// bf16 operands of later GEMMs: streaming (the backward kernels run UPT = 8 or 1)
+template <int UPT>
+SB_DEVINL void st_stream_bf16u(bf16* p, const float (&v)[UPT]) {
+  if constexpr (UPT == 8) {
+    __stcs(reinterpret_cast<uint4*>(p), pack8(v));
+  } else {
+    static_assert(UPT == 1, "st_stream_bf16u: UPT 8 or 1");
+    const unsigned short u = __bfloat16_as_ushort(__float2bfloat16_rn(v[0]));
+    asm volatile("st.global.cs.u16 [%0], %1;" ::"l"(p), "h"(u) : "memory");
+  }
+}
+
 SB_DEVINL void tmem_ld_32x32b_x8(uint32_t taddr, uint32_t (&v)[8]) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
@@ -252,8 +547,163 @@ SB_DEVINL void tmem_ld_32x32b_x8(uint32_t taddr, uint32_t (&v)[8]) {
       : "memory");
 }
 
+// Saved per step by the forward pass for the backward one: r, z, n and hn = W_hn h_{t-1} + b_hn.
+template <int UPT>
+struct GruGates {
+  float r[UPT], z[UPT], n[UPT], hn[UPT];
+};
+// Backward per step: d(pre-activation) of r, z, n and dn * r (also used for their sums over t, b).
+template <int UPT>
+struct GruGrad {
+  float r[UPT], z[UPT], n[UPT], nr[UPT];
+};
+
+// All epilogue threads have published: one arrive per CTA on the direction's grid barrier
+// (release: cumulative over the CTA's writes ordered by bar.sync).
+template <class Params>
+SB_DEVINL void gru_arrive(const Params& p, int step, int tid, unsigned int* ctr, bool skew_probe) {
+  epi_barrier();
+  if (tid == 0) {
+    GRU_STAMP(7);
+    if (skew_probe && p.dbg && step == 20) p.dbg[1024 + blockIdx.x] = gtime();   // skew probe
+    grid_arrive(ctr);
+    GRU_STAMP(9);
+  }
+}
+
+// ---- forward cell ---------------------------------------------------------------------------
+// the input projections of step t do not depend on the recurrence: fetched first
+template <int UPT>
+SB_DEVINL void gru_load_gi(const GruFwdParams& p, int t, int row, int dir, int ju,
+                           float (&gi)[3][UPT]) {
+  const int H = p.H;
+  const float* g = p.gi + ((long long)t * p.Bp + row) * (p.ndir * 3 * H) + dir * 3 * H + ju;
+#pragma unroll
+  for (int gg = 0; gg < 3; ++gg) ldu<UPT>(g + gg * H, gi[gg]);
+}
+template <int UPT>
+SB_DEVINL void gru_cell_fwd(const float (&gi)[3][UPT], const float (&acc)[3][UPT],
+                            const float (&bias)[3][UPT], float (&h)[UPT], GruGates<UPT>& g) {
+#pragma unroll
+  for (int jj = 0; jj < UPT; ++jj) {
+    g.r[jj] = fast_sigmoid(gi[0][jj] + acc[0][jj] + bias[0][jj]);
+    g.z[jj] = fast_sigmoid(gi[1][jj] + acc[1][jj] + bias[1][jj]);
+    g.hn[jj] = acc[2][jj] + bias[2][jj];
+    g.n[jj] = fast_tanh(gi[2][jj] + g.r[jj] * g.hn[jj]);
+    h[jj] = (1.f - g.z[jj]) * g.n[jj] + g.z[jj] * h[jj];
+  }
+}
+// critical path: only the bf16 h_t that the other CTAs gather next step (then gru_arrive)
+template <int UPT>
+SB_DEVINL void gru_publish_fwd(const GruFwdParams& p, int step, int tid, bool active, bf16* dst,
+                               const float (&h)[UPT], unsigned int* ctr, bool skew_probe) {
+  if (active) {
+    st_bf16u<UPT>(dst, h);
+    if (tid == 0) GRU_STAMP(5);
+    fence_proxy_async_global();   // generic writes -> other CTAs' TMA reads
+    if (tid == 0) GRU_STAMP(6);
+  }
+  gru_arrive(p, step, tid, ctr, skew_probe);
+}
+// off the critical path: fp32 state, saved gates
+template <int UPT>
+SB_DEVINL void gru_store_fwd(const GruFwdParams& p, long long m, int dir, int ju,
+                             const float (&h)[UPT], const GruGates<UPT>& g) {
+  const int H = p.H;
+  stu<UPT>(p.y + m * (p.ndir * H) + dir * H + ju, h);
+  if (p.gates) {
+    float* go = p.gates + ((m * p.ndir + dir) * 4) * H + ju;
+    stu<UPT>(go, g.r);
+    stu<UPT>(go + H, g.z);
+    stu<UPT>(go + 2 * H, g.n);
+    stu<UPT>(go + 3 * H, g.hn);
+  }
+}
+
+// ---- backward cell --------------------------------------------------------------------------
+// saved activations of step t (row m), dL/dy and h_{t-1} (row mp): independent of the recurrence,
+// fetched first
+template <int UPT>
+SB_DEVINL void gru_load_bwd(const GruBwdParams& p, long long m, long long mp, bool has_prev,
+                            int dir, int ju, GruGates<UPT>& g, float (&dh)[UPT],
+                            float (&hp)[UPT]) {
+  const int H = p.H, D = p.ndir * H;
+  const float* go = p.gates + ((m * p.ndir + dir) * 4) * H + ju;
+  ldu<UPT>(go, g.r);
+  ldu<UPT>(go + H, g.z);
+  ldu<UPT>(go + 2 * H, g.n);
+  ldu<UPT>(go + 3 * H, g.hn);
+  ldu<UPT>(p.dy + m * D + dir * H + ju, dh);
+  if (has_prev) {
+    ldu<UPT>(p.y + mp * D + dir * H + ju, hp);
+  } else {
+#pragma unroll
+    for (int jj = 0; jj < UPT; ++jj) hp[jj] = 0.f;
+  }
+}
+// dh_rec: in, the part of dL/dh_t that arrived through the recurrence; out, the direct path
+// h_{t-1} -> h_t (the W_hh path is added next step).
+template <int UPT>
+SB_DEVINL void gru_cell_bwd(const GruGates<UPT>& a, const float (&dh)[UPT], const float (&hp)[UPT],
+                            float (&dh_rec)[UPT], GruGrad<UPT>& d, GruGrad<UPT>& db) {
+#pragma unroll
+  for (int jj = 0; jj < UPT; ++jj) {
+    const float g = dh[jj] + dh_rec[jj];
+    d.n[jj] = g * (1.f - a.z[jj]) * (1.f - a.n[jj] * a.n[jj]);
+    d.z[jj] = g * (hp[jj] - a.n[jj]) * a.z[jj] * (1.f - a.z[jj]);
+    d.r[jj] = d.n[jj] * a.hn[jj] * a.r[jj] * (1.f - a.r[jj]);
+    d.nr[jj] = d.n[jj] * a.r[jj];
+    dh_rec[jj] = g * a.z[jj];
+    db.r[jj] += d.r[jj];
+    db.z[jj] += d.z[jj];
+    db.n[jj] += d.n[jj];
+    db.nr[jj] += d.nr[jj];
+  }
+}
+// critical path: the exchange row [dr | dz | dn*r] that every CTA gathers for the next product
+// (x: this thread's units in row `row` of the step's exchange buffer; then gru_arrive)
+template <int UPT>
+SB_DEVINL void gru_publish_bwd(const GruBwdParams& p, int step, int tid, bool active, bf16* x,
+                               const GruGrad<UPT>& d, unsigned int* ctr) {
+  if (step + 1 < p.T) {   // the last step processed has no successor
+    if (active) {
+      st_bf16u<UPT>(x, d.r);
+      st_bf16u<UPT>(x + p.H, d.z);
+      st_bf16u<UPT>(x + 2 * p.H, d.nr);
+      if (tid == 0) GRU_STAMP(5);
+      fence_proxy_async_global();
+      if (tid == 0) GRU_STAMP(6);
+    }
+    gru_arrive(p, step, tid, ctr, false);
+  }
+}
+// off the critical path: operands of the dX / dW GEMMs
+template <int UPT>
+SB_DEVINL void gru_store_bwd(const GruBwdParams& p, long long m, int dir, int ju,
+                             const GruGrad<UPT>& d) {
+  const int H = p.H, K3 = 3 * H;
+  bf16* o = p.dgi + m * (p.ndir * K3) + dir * K3 + ju;
+  st_stream_bf16u<UPT>(o, d.r);
+  st_stream_bf16u<UPT>(o + H, d.z);
+  st_stream_bf16u<UPT>(o + 2 * H, d.n);
+  st_stream_bf16u<UPT>(p.dghn + m * (p.ndir * H) + dir * H + ju, d.nr);
+}
+
 // =============================================================================================
-// forward
+// forward, full gather
+//   * CTA c of direction d owns 16 hidden units j0..j0+15: its 48 rows of W_hh (r,z,n) stay
+//     resident in shared memory (bf16, UMMA K-major SWIZZLE_128B chunks) for all T steps;
+//   * per step every CTA needs ALL of h_{t-1} (bf16, written by the CTAs of its direction in the
+//     previous step).  CTAs form thread-block clusters of up to 4; each CTA fetches 1/CS of the
+//     [Bp x 64] chunks with TMA and MULTICASTS them into the shared memory of all CTAs of its
+//     cluster, so L2 is read once per cluster instead of once per CTA (the un-multicast version
+//     was bound by 64 SMs hammering the same L2 lines: 4 us of a 13 us step);
+//   * one thread issues tcgen05.mma  D[batch(128) x 48] += h_{t-1}[batch x 64] * Wslice[48 x 64]^T
+//     per chunk as its mbarrier completes; accumulators live in TMEM;
+//   * 8 epilogue warps (thread = TMEM lane = batch row, 8 hidden units each) read the
+//     accumulators with tcgen05.ld, apply the gate math in fp32 (h_{t-1} of the thread's own units
+//     stays in registers across steps), publish the bf16 h_t, arrive on the per-direction grid
+//     barrier, and only then write the fp32 state / saved gates.
 // =============================================================================================
 __global__ void __launch_bounds__(GRU_THREADS, 1)
 gru_fwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant__ CUtensorMap tm_d1,
@@ -265,20 +715,15 @@ gru_fwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
   const int j0 = (blockIdx.x % nC) * GRU_HC;
   const int nchunks = (H + 63) / 64;
   constexpr int WCHUNK = 48 * 128;  // 48 rows x 64 bf16
-  const int ring_bytes = p.ring * p.gc * Bp * 128;
-  // the 128-row A read of the last ring slot overruns by (16 KB - stride) into this region
-  const int wbytes = max(nchunks * WCHUNK, 16384 - Bp * 128);
-  const GruSmem s = carve(smem_raw, ring_bytes, wbytes);
+  const GruSmemLayout L = gru_layout_full(Bp, nchunks, 48, p.ring * p.gc * Bp * 128);
+  const GruSmem s = gru_carve(smem_raw, L);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int D = p.ndir * H;
   const CUtensorMap* tm = dir == 0 ? &tm_d0 : &tm_d1;
   const uint32_t crank = cluster_rank(), csize = cluster_size();
 
-  // ---- one-time setup: zero ring + weight region, stage the 48 weight rows, barriers, TMEM ----
-  for (int k = tid; k < (ring_bytes + wbytes) / 16; k += GRU_THREADS)
-    reinterpret_cast<uint4*>(s.ring)[k] = make_uint4(0, 0, 0, 0);
-  __syncthreads();
-  {
+  const uint32_t tmem_base = gru_setup(s, L, tm, 64, csize, [&] {
+    // the 48 weight rows (gate g, unit jj) and their b_hh
     const int pieces_per_row = nchunks * 8;
     for (int k = tid; k < 48 * pieces_per_row; k += GRU_THREADS) {
       const int r = k / pieces_per_row, pc = k % pieces_per_row;
@@ -294,23 +739,7 @@ gru_fwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
       const int g = tid / GRU_HC, jj = tid % GRU_HC;
       s.scratch[tid] = p.bhh[dir * 3 * H + g * H + j0 + jj];
     }
-  }
-  if (tid == 0) {
-    for (int i = 0; i < GRU_MAX_RING; ++i) {
-      mbar_init(&s.full[i], 1);
-      mbar_init(&s.empty[i], csize);
-    }
-    mbar_init(s.accfull, 1);
-    mbar_fence_init();
-    tma_prefetch_desc(tm);
-  }
-  if (warp == 8) tmem_alloc(s.tmem_slot, 64);
-  fence_proxy_async_smem();
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  cluster_sync_all();   // peers' barriers are initialised before anyone multicasts into them
-  const uint32_t tmem_base = *s.tmem_slot;
+  });
   unsigned int* ctr = p.barrier + dir * 32;   // one L2 line per direction
 
   if (warp == 9) {
@@ -350,13 +779,8 @@ gru_fwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
     const bool active = row < Bp;
     for (int step = 0; step < T; ++step) {
       const int t = dir == 0 ? step : (T - 1 - step);
-      // this step's input projections do not depend on the recurrence: fetch them first
       float gi[3][GRU_UPT];
-      if (active) {
-        const float* g = p.gi + ((long long)t * Bp + row) * (p.ndir * 3 * H) + dir * 3 * H + ju;
-#pragma unroll
-        for (int gg = 0; gg < 3; ++gg) ld8(g + gg * H, gi[gg]);
-      }
+      if (active) gru_load_gi(p, t, row, dir, ju, gi);
       float acc[3][GRU_UPT];
       if (step > 0) {
         mbar_wait(s.accfull, (step - 1) & 1);
@@ -380,54 +804,20 @@ gru_fwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
           for (int jj = 0; jj < GRU_UPT; ++jj) acc[gg][jj] = 0.f;
       }
       const long long m = (long long)t * Bp + row;
-      float hn[GRU_UPT], rr[GRU_UPT], zz[GRU_UPT], nn[GRU_UPT];
-      if (active) {
-#pragma unroll
-        for (int jj = 0; jj < GRU_UPT; ++jj) {
-          rr[jj] = fast_sigmoid(gi[0][jj] + acc[0][jj] + bias[0][jj]);
-          zz[jj] = fast_sigmoid(gi[1][jj] + acc[1][jj] + bias[1][jj]);
-          hn[jj] = acc[2][jj] + bias[2][jj];
-          nn[jj] = fast_tanh(gi[2][jj] + rr[jj] * hn[jj]);
-          hprev[jj] = (1.f - zz[jj]) * nn[jj] + zz[jj] * hprev[jj];
-        }
-        // critical path: only the bf16 h_t that the other CTAs gather next step
-        *reinterpret_cast<uint4*>(p.xn + m * D + dir * H + ju) = pack8(hprev);
-        if (tid == 0) GRU_STAMP(5);
-        fence_proxy_async_global();   // generic writes -> other CTAs' TMA reads
-        if (tid == 0) GRU_STAMP(6);
-      }
-      epi_barrier();
-      if (tid == 0) {
-        GRU_STAMP(7);
-        grid_arrive(ctr);          // release: cumulative over the CTA's writes ordered by bar.sync
-        GRU_STAMP(9);
-      }
-      // off the critical path: fp32 state, saved gates
-      if (active) {
-        st8(p.y + m * D + dir * H + ju, hprev);
-        if (p.gates) {
-          float* go = p.gates + ((m * p.ndir + dir) * 4) * H + ju;
-          st8(go, rr);
-          st8(go + H, zz);
-          st8(go + 2 * H, nn);
-          st8(go + 3 * H, hn);
-        }
-      }
+      GruGates<GRU_UPT> g;
+      if (active) gru_cell_fwd(gi, acc, bias, hprev, g);
+      gru_publish_fwd(p, step, tid, active, p.xn + m * D + dir * H + ju, hprev, ctr, false);
+      if (active) gru_store_fwd(p, m, dir, ju, hprev, g);
       if (tid == 0) GRU_STAMP(10);
     }
   }
-
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();   // no CTA leaves while peers may still signal its barriers
-  if (warp == 8) {
-    tc_fence_after_sync();
-    tmem_dealloc(tmem_base, 64);
-  }
+  gru_teardown(tmem_base, 64);
 }
 
 // =============================================================================================
-// backward (reverse of the forward time order of each direction)
+// backward, full gather (reverse of the forward time order of each direction): the structure of
+// gru_fwd_kernel with W_hh^T resident (16 rows x 3H) and the all-gather over the pre-activation
+// gradients dgh_t (batch x 3H).
 // =============================================================================================
 __global__ void __launch_bounds__(GRU_THREADS, 1)
 gru_bwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant__ CUtensorMap tm_d1,
@@ -440,18 +830,13 @@ gru_bwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
   const int K3 = 3 * H;
   const int nchunks = (K3 + 63) / 64;
   constexpr int WCHUNK = 16 * 128;  // 16 rows x 64 bf16
-  const int ring_bytes = p.ring * p.gc * Bp * 128;
-  const int wbytes = max(nchunks * WCHUNK, 16384 - Bp * 128);
-  const GruSmem s = carve(smem_raw, ring_bytes, wbytes);
+  const GruSmemLayout L = gru_layout_full(Bp, nchunks, 16, p.ring * p.gc * Bp * 128);
+  const GruSmem s = gru_carve(smem_raw, L);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int D = p.ndir * H;
   const CUtensorMap* tm = dir == 0 ? &tm_d0 : &tm_d1;
   const uint32_t crank = cluster_rank(), csize = cluster_size();
 
-  for (int k = tid; k < (ring_bytes + wbytes) / 16; k += GRU_THREADS)
-    reinterpret_cast<uint4*>(s.ring)[k] = make_uint4(0, 0, 0, 0);
-  __syncthreads();
-  {
+  const uint32_t tmem_base = gru_setup(s, L, tm, 32, csize, [&] {
     // resident operand: rows = the 16 hidden units j0..j0+15 of W_hh^T, K = 3H.  W_hh is read as
     // stored ([3H][H]: 32 contiguous bytes per k) and transposed on the way into shared memory
     for (int k = tid; k < K3 * 2; k += GRU_THREADS) {
@@ -465,23 +850,7 @@ gru_bwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
         *reinterpret_cast<unsigned short*>(
             chunk + sw128_offset((uint32_t)(half * 8 + q), (uint32_t)((kk & 63) >> 3))) = e[q];
     }
-  }
-  if (tid == 0) {
-    for (int i = 0; i < GRU_MAX_RING; ++i) {
-      mbar_init(&s.full[i], 1);
-      mbar_init(&s.empty[i], csize);
-    }
-    mbar_init(s.accfull, 1);
-    mbar_fence_init();
-    tma_prefetch_desc(tm);
-  }
-  if (warp == 8) tmem_alloc(s.tmem_slot, 32);
-  fence_proxy_async_smem();
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  cluster_sync_all();
-  const uint32_t tmem_base = *s.tmem_slot;
+  });
   unsigned int* ctr = p.barrier + dir * 32;   // one L2 line per direction
 
   if (warp == 9) {
@@ -507,10 +876,10 @@ gru_bwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
     const int ju = j0 + uh * GRU_UPT;
     const bool active = row < Bp;
     float dh_rec[GRU_UPT];   // dL/dh_t arriving through the recurrence (own units)
-    float db_r[GRU_UPT], db_z[GRU_UPT], db_n[GRU_UPT], db_hn[GRU_UPT];
+    GruGrad<GRU_UPT> db;
 #pragma unroll
     for (int jj = 0; jj < GRU_UPT; ++jj) {
-      dh_rec[jj] = 0.f; db_r[jj] = 0.f; db_z[jj] = 0.f; db_n[jj] = 0.f; db_hn[jj] = 0.f;
+      dh_rec[jj] = 0.f; db.r[jj] = 0.f; db.z[jj] = 0.f; db.n[jj] = 0.f; db.nr[jj] = 0.f;
     }
 
     for (int step = 0; step < T; ++step) {
@@ -520,22 +889,9 @@ gru_bwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
       const bool has_prev = dir == 0 ? (t > 0) : (t < T - 1);
       bf16* xb = p.xchg + ((long long)(dir * 2 + (step & 1)) * Bp) * K3;
       const long long m = (long long)t * Bp + row;
-      // ---- saved activations of this step: independent of the recurrence, fetched first ----
-      float rr[GRU_UPT], zz[GRU_UPT], nn[GRU_UPT], hn[GRU_UPT], dh[GRU_UPT], hp[GRU_UPT];
-      if (active) {
-        const float* go = p.gates + ((m * p.ndir + dir) * 4) * H + ju;
-        ld8(go, rr);
-        ld8(go + H, zz);
-        ld8(go + 2 * H, nn);
-        ld8(go + 3 * H, hn);
-        ld8(p.dy + m * D + dir * H + ju, dh);
-        if (has_prev) {
-          ld8(p.y + ((long long)tp * Bp + row) * D + dir * H + ju, hp);
-        } else {
-#pragma unroll
-          for (int jj = 0; jj < GRU_UPT; ++jj) hp[jj] = 0.f;
-        }
-      }
+      GruGates<GRU_UPT> a;
+      float dh[GRU_UPT], hp[GRU_UPT];
+      if (active) gru_load_bwd(p, m, (long long)tp * Bp + row, has_prev, dir, ju, a, dh, hp);
       // ---- recurrent part of dL/dh_t: product issued in the previous step ----
       if (step > 0) {
         mbar_wait(s.accfull, (step - 1) & 1);
@@ -549,48 +905,10 @@ gru_bwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
 #pragma unroll
         for (int jj = 0; jj < GRU_UPT; ++jj) dh_rec[jj] += __uint_as_float(v[jj]);
       }
-      float dr[GRU_UPT], dz[GRU_UPT], dn[GRU_UPT], dnr[GRU_UPT];
-      if (active) {
-#pragma unroll
-        for (int jj = 0; jj < GRU_UPT; ++jj) {
-          const float g = dh[jj] + dh_rec[jj];
-          dn[jj] = g * (1.f - zz[jj]) * (1.f - nn[jj] * nn[jj]);
-          dz[jj] = g * (hp[jj] - nn[jj]) * zz[jj] * (1.f - zz[jj]);
-          dr[jj] = dn[jj] * hn[jj] * rr[jj] * (1.f - rr[jj]);
-          dnr[jj] = dn[jj] * rr[jj];
-          dh_rec[jj] = g * zz[jj];      // direct path h_{t-1} -> h_t; the W_hh path is added next step
-          db_r[jj] += dr[jj];
-          db_z[jj] += dz[jj];
-          db_n[jj] += dn[jj];
-          db_hn[jj] += dnr[jj];
-        }
-        // critical path: the exchange rows [dr | dz | dn*r] every CTA gathers for the product
-        if (step + 1 < T) {
-          bf16* x = xb + (long long)row * K3 + ju;
-          *reinterpret_cast<uint4*>(x) = pack8(dr);
-          *reinterpret_cast<uint4*>(x + H) = pack8(dz);
-          *reinterpret_cast<uint4*>(x + 2 * H) = pack8(dnr);
-          if (tid == 0) GRU_STAMP(5);
-          fence_proxy_async_global();
-          if (tid == 0) GRU_STAMP(6);
-        }
-      }
-      if (step + 1 < T) {
-        epi_barrier();
-        if (tid == 0) {
-          GRU_STAMP(7);
-          grid_arrive(ctr);
-          GRU_STAMP(9);
-        }
-      }
-      // ---- off the critical path: operands of the dX / dW GEMMs ----
-      if (active) {
-        bf16* o = p.dgi + m * (p.ndir * K3) + dir * K3 + ju;
-        st_stream_u4(o, pack8(dr));
-        st_stream_u4(o + H, pack8(dz));
-        st_stream_u4(o + 2 * H, pack8(dn));
-        st_stream_u4(p.dghn + m * D + dir * H + ju, pack8(dnr));
-      }
+      GruGrad<GRU_UPT> d;
+      if (active) gru_cell_bwd(a, dh, hp, dh_rec, d, db);
+      gru_publish_bwd(p, step, tid, active, xb + (long long)row * K3 + ju, d, ctr);
+      if (active) gru_store_bwd(p, m, dir, ju, d);
       if (tid == 0) GRU_STAMP(10);
     }
     // ---- bias gradients: reduce the per-batch-row partial sums over the CTA ----
@@ -600,10 +918,10 @@ gru_bwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
     epi_barrier();
 #pragma unroll
     for (int jj = 0; jj < GRU_UPT; ++jj) {
-      const float a = warp_sum(active ? db_r[jj] : 0.f);
-      const float b = warp_sum(active ? db_z[jj] : 0.f);
-      const float c = warp_sum(active ? db_n[jj] : 0.f);
-      const float d = warp_sum(active ? db_hn[jj] : 0.f);
+      const float a = warp_sum(active ? db.r[jj] : 0.f);
+      const float b = warp_sum(active ? db.z[jj] : 0.f);
+      const float c = warp_sum(active ? db.n[jj] : 0.f);
+      const float d = warp_sum(active ? db.nr[jj] : 0.f);
       if (lane == 0) {
         atomicAdd(&red[uh * GRU_UPT + jj], a);
         atomicAdd(&red[16 + uh * GRU_UPT + jj], b);
@@ -619,14 +937,7 @@ gru_bwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
       atomicAdd(p.dbhh + idx, g < 2 ? red[tid] : red[48 + jj]);
     }
   }
-
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 8) {
-    tc_fence_after_sync();
-    tmem_dealloc(tmem_base, 32);
-  }
+  gru_teardown(tmem_base, 32);
 }
 
 // =============================================================================================
@@ -637,55 +948,13 @@ gru_bwd_kernel(const __grid_constant__ CUtensorMap tm_d0, const __grid_constant_
 // the gather alone costs ~9 us of the 15.8 us step.  Here CTA r of a cluster contracts only the
 // r-th QUARTER of the K = 3H dimension, for all 64 units of its cluster:
 //     D_r[batch x 64] = dgh_t[:, quarter r] * W_hh[quarter r, 64 units]          (96 KB gathered)
-// and the four partial products are reduce-scattered through distributed shared memory: each
-// epilogue thread pushes the three 8-float slices that belong to peer CTAs with st.shared::cluster
-// and arrives (release.cluster) on the peer's mbarrier; the owner adds the three slices it received
-// to its own.  12 KB of DSMEM traffic replaces 288 KB of L2 reads per CTA per step.
+// and the four partial products are reduce-scattered through distributed shared memory: for each
+// peer in turn, the epilogue stages the 16 columns that belong to it in local shared memory and
+// sends them with ONE bulk copy into the peer's receive buffer, completing on the peer's mbarrier;
+// the owner adds the three slices it received to its own.  12 KB of DSMEM traffic replaces 288 KB
+// of L2 reads per CTA per step.
 // Requires cluster size 4, H % 256 == 0.
 // =============================================================================================
-static constexpr int KS = 4;
-
-SB_DEVINL uint32_t mapa_shared(uint32_t local_addr, uint32_t peer) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_addr), "r"(peer));
-  return r;
-}
-SB_DEVINL void st_cluster_f4(uint32_t raddr, float4 v) {
-  asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(raddr), "f"(v.x),
-               "f"(v.y), "f"(v.z), "f"(v.w)
-               : "memory");
-}
-SB_DEVINL void mbar_arrive_remote_release(uint32_t raddr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(raddr)
-               : "memory");
-}
-SB_DEVINL void mbar_wait_acquire_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0, ok = 0;
-  while (!ok) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred P;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, P;\n\t"
-        "}\n"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    if (!ok && ++spins > SB_SPIN_LIMIT) __trap();
-  }
-}
-
-// bulk copy from this CTA's shared memory into a PEER's shared memory (DSMEM through the copy
-// engine), completing `bytes` on the peer's mbarrier.  Measured: pushing the reduce-scatter
-// slices with per-thread st.shared::cluster took 4.1 us for 36 KB (~9 KB/us per SM).
-SB_DEVINL void bulk_s2peer(uint32_t peer_dst, const void* local_src, uint32_t bytes,
-                           uint32_t peer_bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-      ::"r"(peer_dst), "r"(smem_u32(local_src)), "r"(bytes), "r"(peer_bar)
-      : "memory");
-}
-
 __global__ void __launch_bounds__(GRU_THREADS, 1)
 gru_bwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
                   const __grid_constant__ CUtensorMap tm_d1, const GruBwdParams p) {
@@ -700,96 +969,30 @@ gru_bwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
   const int K3 = 3 * H;
   const int KQ = K3 / KS;                             // this CTA's share of the contraction
   const int nchunks = KQ / 64;
-  constexpr int WCHUNK = 64 * 128;                    // 64 rows (units) x 64 bf16
   const int stride = Bp * 128;
-  const int ring_bytes = nchunks * stride;            // the whole quarter is resident
-  const int wbytes = nchunks * WCHUNK;
-  // carve: ring | weights | recv | barriers
-  uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
-                                             ~static_cast<uintptr_t>(1023));
-  uint8_t* ring = base;
-  uint8_t* wtile = ring + ring_bytes;
-  float* recv = reinterpret_cast<float*>(wtile + wbytes);          // [KS][Bp][16] from peer src
-  float* stage = recv + KS * Bp * 16;                              // [KS][Bp][16] for peer dst
-  uint64_t* bars = reinterpret_cast<uint64_t*>(stage + KS * Bp * 16);
-  uint64_t* full = bars;          // [4] groups
-  uint64_t* accfull = bars + 4;
-  uint64_t* recvbar = bars + 5;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 6);
+  const GruSmemLayout L = gru_layout_bwd_ks(Bp, H);
+  const GruSmem s = gru_carve(smem_raw, L);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int D = p.ndir * H;
   const CUtensorMap* tm = dir == 0 ? &tm_d0 : &tm_d1;
-  const int gc = (nchunks % 4 == 0) ? 4 : ((nchunks % 3 == 0) ? 3 : ((nchunks % 2 == 0) ? 2 : 1));
-  const int ngroups = nchunks / gc;                   // <= 4 for H <= 1024 ... checked on host
+  const int gc = gru_group_chunks(nchunks);
+  const int ngroups = nchunks / gc;                   // <= GRU_KS_BWD_GROUPS: checked on the host
 
-  for (int k = tid; k < (ring_bytes + wbytes + 2 * KS * Bp * 64) / 16; k += GRU_THREADS)
-    reinterpret_cast<uint4*>(base)[k] = make_uint4(0, 0, 0, 0);
-  __syncthreads();
-  {
-    // resident operand: rows = the cluster's 64 units of W_hh^T, columns = this CTA's K quarter.
-    // W_hh is read as stored ([3H][H]: the cluster's 64 units are 128 contiguous bytes of row k)
-    // and transposed on the way into shared memory (once per launch)
-    for (int k = tid; k < KQ * 8; k += GRU_THREADS) {
-      const int kl = k >> 3, piece = k & 7;       // local k, 8-unit piece of the 64 units
-      const uint4 v = *reinterpret_cast<const uint4*>(
-          p.whh + ((long long)dir * K3 + (long long)crank * KQ + kl) * H + k0c + piece * 8);
-      const unsigned short* e = reinterpret_cast<const unsigned short*>(&v);
-      uint8_t* chunk = wtile + (kl >> 6) * WCHUNK + (kl & 7) * 2;
-#pragma unroll
-      for (int q = 0; q < 8; ++q)
-        *reinterpret_cast<unsigned short*>(
-            chunk + sw128_offset((uint32_t)(piece * 8 + q), (uint32_t)((kl & 63) >> 3))) = e[q];
-    }
-  }
-  if (tid == 0) {
-    for (int i = 0; i < 4; ++i) mbar_init(&full[i], 1);
-    mbar_init(accfull, 1);
-    mbar_init(recvbar, 1);   // one local arrive.expect_tx per step; the peers' copies complete_tx
-    mbar_fence_init();
-    tma_prefetch_desc(tm);
-  }
-  if (warp == 8) tmem_alloc(tmem_slot, 64);
-  fence_proxy_async_smem();
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  cluster_sync_all();
-  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_base =
+      gru_setup(s, L, tm, 64, KS, [&] { ks_stage_whh_t(s.wtile, p.whh, H, dir, k0c, crank); });
   unsigned int* ctr = p.barrier + dir * 32;   // one L2 line per direction
 
   if (warp == 9) {
     if (lane == 0) {
       for (int step = 0; step + 1 < T; ++step) {
         grid_wait(ctr, (unsigned int)nC * (step + 1));   // dgh of this step is complete
-        for (int g = 0; g < ngroups; ++g) {
-          mbar_expect_tx(&full[g], (uint32_t)(stride * gc));
-          for (int i = 0; i < gc; ++i) {
-            const int c = g * gc + i;
-            tma_load_2d(ring + c * stride, tm, &full[g], (int)crank * KQ + c * 64,
-                        (step & 1) * Bp);
-          }
-        }
+        ks_gather_bwd(s, tm, stride, ngroups, gc, (int)crank * KQ, (step & 1) * Bp);
       }
     }
   } else if (warp == 8) {
     if (lane == 0) {
-      constexpr uint32_t idesc = umma_idesc_bf16_f32(128, 64);
-      for (int step = 0; step + 1 < T; ++step) {
-        for (int g = 0; g < ngroups; ++g) {
-          mbar_wait(&full[g], step & 1);
-          tc_fence_after_sync();
-          for (int i = 0; i < gc; ++i) {
-            const int c = g * gc + i;
-            const uint64_t da = umma_desc_sw128_kmajor(smem_u32(ring + c * stride));
-            const uint64_t db = umma_desc_sw128_kmajor(smem_u32(wtile + c * WCHUNK));
-#pragma unroll
-            for (int kk = 0; kk < 4; ++kk)
-              umma_bf16_ss(tmem_base, da + (uint64_t)(kk * 2), db + (uint64_t)(kk * 2), idesc,
-                           (c > 0 || kk > 0) ? 1u : 0u);
-          }
-        }
-        umma_commit(accfull);
-      }
+      for (int step = 0; step + 1 < T; ++step)
+        ks_mma_bwd(s, tmem_base, stride, ngroups, gc, 64 * 128, umma_idesc_bf16_f32(128, 64),
+                   false, step & 1);
     }
   } else {
     const int row = (warp & 3) * 32 + lane;
@@ -797,10 +1000,10 @@ gru_bwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
     const int ju = j0 + uh * GRU_UPT;
     const bool active = row < Bp;
     float dh_rec[GRU_UPT];
-    float db_r[GRU_UPT], db_z[GRU_UPT], db_n[GRU_UPT], db_hn[GRU_UPT];
+    GruGrad<GRU_UPT> db;
 #pragma unroll
     for (int jj = 0; jj < GRU_UPT; ++jj) {
-      dh_rec[jj] = 0.f; db_r[jj] = 0.f; db_z[jj] = 0.f; db_n[jj] = 0.f; db_hn[jj] = 0.f;
+      dh_rec[jj] = 0.f; db.r[jj] = 0.f; db.z[jj] = 0.f; db.n[jj] = 0.f; db.nr[jj] = 0.f;
     }
 
     for (int step = 0; step < T; ++step) {
@@ -809,28 +1012,16 @@ gru_bwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
       const bool has_prev = dir == 0 ? (t > 0) : (t < T - 1);
       bf16* xb = p.xchg + ((long long)(dir * 2 + (step & 1)) * Bp) * K3;
       const long long m = (long long)t * Bp + row;
-      float rr[GRU_UPT], zz[GRU_UPT], nn[GRU_UPT], hn[GRU_UPT], dh[GRU_UPT], hp[GRU_UPT];
-      if (active) {
-        const float* go = p.gates + ((m * p.ndir + dir) * 4) * H + ju;
-        ld8(go, rr);
-        ld8(go + H, zz);
-        ld8(go + 2 * H, nn);
-        ld8(go + 3 * H, hn);
-        ld8(p.dy + m * D + dir * H + ju, dh);
-        if (has_prev) {
-          ld8(p.y + ((long long)tp * Bp + row) * D + dir * H + ju, hp);
-        } else {
-#pragma unroll
-          for (int jj = 0; jj < GRU_UPT; ++jj) hp[jj] = 0.f;
-        }
-      }
+      GruGates<GRU_UPT> a;
+      float dh[GRU_UPT], hp[GRU_UPT];
+      if (active) gru_load_bwd(p, m, (long long)tp * Bp + row, has_prev, dir, ju, a, dh, hp);
       // ---- recurrent part of dL/dh_t: reduce-scatter of the four partial products ----
       if (step > 0) {
-        mbar_wait(accfull, (step - 1) & 1);
+        mbar_wait(s.accfull, (step - 1) & 1);
         if (tid == 0) GRU_STAMP(3);
         tc_fence_after_sync();
         float own[GRU_UPT];
-        if (tid == 0) mbar_expect_tx(recvbar, (uint32_t)((KS - 1) * Bp * 16 * 4));
+        if (tid == 0) mbar_expect_tx(s.recvbar, (uint32_t)((KS - 1) * Bp * 16 * 4));
         // the peers' slices first, each staged and sent as soon as it is complete (see
         // gru_fwd_ks_kernel); the own slice last
 #pragma unroll 1
@@ -845,7 +1036,7 @@ gru_bwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
             for (int jj = 0; jj < GRU_UPT; ++jj) own[jj] = __uint_as_float(v[jj]);
           } else {
             if (active) {
-              float4* sp = reinterpret_cast<float4*>(stage + ((size_t)pr * Bp + row) * 16 +
+              float4* sp = reinterpret_cast<float4*>(s.stage + ((size_t)pr * Bp + row) * 16 +
                                                      uh * GRU_UPT);
               sp[0] = make_float4(__uint_as_float(v[0]), __uint_as_float(v[1]),
                                   __uint_as_float(v[2]), __uint_as_float(v[3]));
@@ -855,14 +1046,14 @@ gru_bwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
             fence_proxy_async_smem();
             epi_barrier();
             if (tid == 0)
-              bulk_s2peer(mapa_shared(smem_u32(recv + (size_t)crank * Bp * 16), pr),
-                          stage + (size_t)pr * Bp * 16, (uint32_t)(Bp * 16 * 4),
-                          mapa_shared(smem_u32(recvbar), pr));
+              bulk_s2peer(mapa_shared(smem_u32(s.recv + (size_t)crank * Bp * 16), pr),
+                          s.stage + (size_t)pr * Bp * 16, (uint32_t)(Bp * 16 * 4),
+                          mapa_shared(smem_u32(s.recvbar), pr));
           }
         }
         tc_fence_before_sync();
         if (tid == 0) GRU_STAMP(4);
-        mbar_wait(recvbar, (step - 1) & 1);
+        mbar_wait(s.recvbar, (step - 1) & 1);
 #pragma unroll
         for (int jj = 0; jj < GRU_UPT; ++jj) dh_rec[jj] += own[jj];
         if (active) {
@@ -870,61 +1061,25 @@ gru_bwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
           for (int src = 0; src < KS; ++src) {
             if ((uint32_t)src == crank) continue;
             const float4* rp = reinterpret_cast<const float4*>(
-                recv + ((size_t)src * Bp + row) * 16 + uh * GRU_UPT);
+                s.recv + ((size_t)src * Bp + row) * 16 + uh * GRU_UPT);
             const float4 a = rp[0], b = rp[1];
             dh_rec[0] += a.x; dh_rec[1] += a.y; dh_rec[2] += a.z; dh_rec[3] += a.w;
             dh_rec[4] += b.x; dh_rec[5] += b.y; dh_rec[6] += b.z; dh_rec[7] += b.w;
           }
         }
       }
-      float dr[GRU_UPT], dz[GRU_UPT], dn[GRU_UPT], dnr[GRU_UPT];
-      if (active) {
-#pragma unroll
-        for (int jj = 0; jj < GRU_UPT; ++jj) {
-          const float g = dh[jj] + dh_rec[jj];
-          dn[jj] = g * (1.f - zz[jj]) * (1.f - nn[jj] * nn[jj]);
-          dz[jj] = g * (hp[jj] - nn[jj]) * zz[jj] * (1.f - zz[jj]);
-          dr[jj] = dn[jj] * hn[jj] * rr[jj] * (1.f - rr[jj]);
-          dnr[jj] = dn[jj] * rr[jj];
-          dh_rec[jj] = g * zz[jj];
-          db_r[jj] += dr[jj];
-          db_z[jj] += dz[jj];
-          db_n[jj] += dn[jj];
-          db_hn[jj] += dnr[jj];
-        }
-        if (step + 1 < T) {
-          bf16* x = xb + (long long)row * K3 + ju;
-          *reinterpret_cast<uint4*>(x) = pack8(dr);
-          *reinterpret_cast<uint4*>(x + H) = pack8(dz);
-          *reinterpret_cast<uint4*>(x + 2 * H) = pack8(dnr);
-          if (tid == 0) GRU_STAMP(5);
-          fence_proxy_async_global();
-          if (tid == 0) GRU_STAMP(6);
-        }
-      }
-      if (step + 1 < T) {
-        epi_barrier();
-        if (tid == 0) {
-          GRU_STAMP(7);
-          grid_arrive(ctr);
-          GRU_STAMP(9);
-        }
-      }
-      if (active) {
-        bf16* o = p.dgi + m * (p.ndir * K3) + dir * K3 + ju;
-        st_stream_u4(o, pack8(dr));
-        st_stream_u4(o + H, pack8(dz));
-        st_stream_u4(o + 2 * H, pack8(dn));
-        st_stream_u4(p.dghn + m * D + dir * H + ju, pack8(dnr));
-      }
+      GruGrad<GRU_UPT> d;
+      if (active) gru_cell_bwd(a, dh, hp, dh_rec, d, db);
+      gru_publish_bwd(p, step, tid, active, xb + (long long)row * K3 + ju, d, ctr);
+      if (active) gru_store_bwd(p, m, dir, ju, d);
       if (tid == 0) GRU_STAMP(10);
     }
 #pragma unroll
     for (int jj = 0; jj < GRU_UPT; ++jj) {
-      const float a = warp_sum(active ? db_r[jj] : 0.f);
-      const float b = warp_sum(active ? db_z[jj] : 0.f);
-      const float c = warp_sum(active ? db_n[jj] : 0.f);
-      const float d = warp_sum(active ? db_hn[jj] : 0.f);
+      const float a = warp_sum(active ? db.r[jj] : 0.f);
+      const float b = warp_sum(active ? db.z[jj] : 0.f);
+      const float c = warp_sum(active ? db.n[jj] : 0.f);
+      const float d = warp_sum(active ? db.nr[jj] : 0.f);
       if (lane == 0) {
         const int bi = dir * K3 + ju + jj;
         atomicAdd(p.dbih + bi, a);
@@ -936,14 +1091,7 @@ gru_bwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
       }
     }
   }
-
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 8) {
-    tc_fence_after_sync();
-    tmem_dealloc(tmem_base, 64);
-  }
+  gru_teardown(tmem_base, 64);
 }
 
 // =============================================================================================
@@ -980,30 +1128,13 @@ gru_fwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
   constexpr int WCHUNK = NCOL * 128;                  // 192 rows x 64 bf16
   constexpr int RW = 3 * GRU_HC;                      // 48 floats received per row and peer
   const int stride = Bp * 128;
-  const int ring_bytes = nchunks * stride;            // the whole quarter is resident
-  const int wbytes = nchunks * WCHUNK;
-  // carve: ring | weights | recv | barriers.  (The 128-row A read of the last chunk runs past the
-  // ring into the weights: finite data, rows >= Bp are never used.)
-  uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
-                                             ~static_cast<uintptr_t>(1023));
-  uint8_t* ring = base;
-  uint8_t* wtile = ring + ring_bytes;
-  float* recv = reinterpret_cast<float*>(wtile + wbytes);          // [KS][Bp][48] from peer src
-  float* stage = recv + KS * Bp * RW;                              // [KS][Bp][48] for peer dst
-  uint64_t* bars = reinterpret_cast<uint64_t*>(stage + KS * Bp * RW);
-  uint64_t* full = bars;
-  uint64_t* accfull = bars + 1;
-  uint64_t* recvbar = bars + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3);
-  float* bias_s = reinterpret_cast<float*>(bars + 4);             // [48]
+  const GruSmemLayout L = gru_layout_fwd_ks(Bp, H);
+  const GruSmem s = gru_carve(smem_raw, L);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int D = p.ndir * H;
   const CUtensorMap* tm = dir == 0 ? &tm_d0 : &tm_d1;
 
-  for (int k = tid; k < (ring_bytes + wbytes + 2 * KS * Bp * RW * 4) / 16; k += GRU_THREADS)
-    reinterpret_cast<uint4*>(base)[k] = make_uint4(0, 0, 0, 0);
-  __syncthreads();
-  {
+  const uint32_t tmem_base = gru_setup(s, L, tm, 256, KS, [&] {
     // resident operand: rows = (gate, unit of the cluster), columns = this CTA's K quarter
     const int pieces_per_row = nchunks * 8;
     for (int k = tid; k < NCOL * pieces_per_row; k += GRU_THREADS) {
@@ -1012,27 +1143,13 @@ gru_fwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
       const uint4 v = *reinterpret_cast<const uint4*>(
           p.whh + ((long long)dir * 3 * H + (long long)g * H + k0c + u) * H + (long long)crank * KQ +
           pc * 8);
-      *reinterpret_cast<uint4*>(wtile + (pc >> 3) * WCHUNK + sw128_offset(r, pc & 7)) = v;
+      *reinterpret_cast<uint4*>(s.wtile + (pc >> 3) * WCHUNK + sw128_offset(r, pc & 7)) = v;
     }
     if (tid < RW) {
       const int g = tid / GRU_HC, jj = tid % GRU_HC;
-      bias_s[tid] = p.bhh[dir * 3 * H + g * H + j0 + jj];
+      s.scratch[tid] = p.bhh[dir * 3 * H + g * H + j0 + jj];
     }
-  }
-  if (tid == 0) {
-    mbar_init(full, 1);
-    mbar_init(accfull, 1);
-    mbar_init(recvbar, 1);   // one local arrive.expect_tx per step; the peers' copies complete_tx
-    mbar_fence_init();
-    tma_prefetch_desc(tm);
-  }
-  if (warp == 8) tmem_alloc(tmem_slot, 256);
-  fence_proxy_async_smem();
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  cluster_sync_all();
-  const uint32_t tmem_base = *tmem_slot;
+  });
   unsigned int* ctr = p.barrier + dir * 32;   // one L2 line per direction
 
   if (warp == 9) {
@@ -1044,9 +1161,7 @@ gru_fwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
         grid_wait(ctr, (unsigned int)nC * step);   // all CTAs published h_{tp}
         GRU_STAMP(0);
         if (p.dbg && step == 21) p.dbg[1024 + 256 + blockIdx.x] = gtime();   // skew probe
-        mbar_expect_tx(full, (uint32_t)(stride * nchunks));
-        for (int c = 0; c < nchunks; ++c)
-          tma_load_2d(ring + c * stride, tm, full, (int)crank * KQ + c * 64, tp * Bp);
+        ks_gather_fwd(s, tm, stride, nchunks, (int)crank * KQ, tp * Bp);
         GRU_STAMP(1);
       }
     }
@@ -1055,17 +1170,7 @@ gru_fwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
     if (lane == 0) {
       constexpr uint32_t idesc = umma_idesc_bf16_f32(128, NCOL);
       for (int step = 1; step < T; ++step) {
-        mbar_wait(full, (step - 1) & 1);
-        tc_fence_after_sync();
-        for (int c = 0; c < nchunks; ++c) {
-          const uint64_t da = umma_desc_sw128_kmajor(smem_u32(ring + c * stride));
-          const uint64_t db = umma_desc_sw128_kmajor(smem_u32(wtile + c * WCHUNK));
-#pragma unroll
-          for (int kk = 0; kk < 4; ++kk)
-            umma_bf16_ss(tmem_base, da + (uint64_t)(kk * 2), db + (uint64_t)(kk * 2), idesc,
-                         (c > 0 || kk > 0) ? 1u : 0u);
-        }
-        umma_commit(accfull);
+        ks_mma_fwd(s, tmem_base, stride, nchunks, WCHUNK, idesc, false, (step - 1) & 1);
         GRU_STAMP(2);
       }
     }
@@ -1082,30 +1187,26 @@ gru_fwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
 #pragma unroll
     for (int g = 0; g < 3; ++g)
 #pragma unroll
-      for (int jj = 0; jj < GRU_UPT; ++jj) bias[g][jj] = bias_s[g * GRU_HC + uh * GRU_UPT + jj];
+      for (int jj = 0; jj < GRU_UPT; ++jj) bias[g][jj] = s.scratch[g * GRU_HC + uh * GRU_UPT + jj];
 
     for (int step = 0; step < T; ++step) {
       const int t = dir == 0 ? step : (T - 1 - step);
       float gi[3][GRU_UPT];
-      if (active) {
-        const float* g = p.gi + ((long long)t * Bp + row) * (p.ndir * 3 * H) + dir * 3 * H + ju;
-#pragma unroll
-        for (int gg = 0; gg < 3; ++gg) ld8(g + gg * H, gi[gg]);
-      }
+      if (active) gru_load_gi(p, t, row, dir, ju, gi);
       float acc[3][GRU_UPT];
 #pragma unroll
       for (int gg = 0; gg < 3; ++gg)
 #pragma unroll
         for (int jj = 0; jj < GRU_UPT; ++jj) acc[gg][jj] = 0.f;
       if (step > 0) {
-        mbar_wait(accfull, (step - 1) & 1);
+        mbar_wait(s.accfull, (step - 1) & 1);
         if (tid == 0) GRU_STAMP(3);
         tc_fence_after_sync();
         // ---- reduce-scatter of the four partial products.  The three slices that belong to
         // the peers go first, one at a time: TMEM -> registers -> local staging -> (named barrier)
         // -> ONE bulk copy into the peer's receive buffer, so the first copy is in flight while
         // the next slice is still being staged; the CTA's own slice is read last ----
-        if (tid == 0) mbar_expect_tx(recvbar, (uint32_t)((KS - 1) * Bp * RW * 4));
+        if (tid == 0) mbar_expect_tx(s.recvbar, (uint32_t)((KS - 1) * Bp * RW * 4));
 #pragma unroll 1
         for (int q = 1; q <= KS; ++q) {
           const uint32_t pr = (crank + (uint32_t)q) % KS;      // q == KS: own slice
@@ -1122,7 +1223,7 @@ gru_fwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
               for (int jj = 0; jj < GRU_UPT; ++jj) acc[gg][jj] = __uint_as_float(v[gg][jj]);
           } else {
             if (active) {
-              float* sp = stage + ((size_t)pr * Bp + row) * RW + uh * GRU_UPT;
+              float* sp = s.stage + ((size_t)pr * Bp + row) * RW + uh * GRU_UPT;
 #pragma unroll
               for (int gg = 0; gg < 3; ++gg) {
                 float4* o = reinterpret_cast<float4*>(sp + gg * GRU_HC);
@@ -1135,19 +1236,19 @@ gru_fwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
             fence_proxy_async_smem();   // generic st.shared -> the copy engine's (async proxy) reads
             epi_barrier();              // this peer's slice is completely staged
             if (tid == 0)
-              bulk_s2peer(mapa_shared(smem_u32(recv + (size_t)crank * Bp * RW), pr),
-                          stage + (size_t)pr * Bp * RW, (uint32_t)(Bp * RW * 4),
-                          mapa_shared(smem_u32(recvbar), pr));
+              bulk_s2peer(mapa_shared(smem_u32(s.recv + (size_t)crank * Bp * RW), pr),
+                          s.stage + (size_t)pr * Bp * RW, (uint32_t)(Bp * RW * 4),
+                          mapa_shared(smem_u32(s.recvbar), pr));
           }
         }
         tc_fence_before_sync();
         if (tid == 0) GRU_STAMP(4);
-        mbar_wait(recvbar, (step - 1) & 1);
+        mbar_wait(s.recvbar, (step - 1) & 1);
         if (active) {
 #pragma unroll
           for (int src = 0; src < KS; ++src) {
             if ((uint32_t)src == crank) continue;
-            const float* rp = recv + ((size_t)src * Bp + row) * RW + uh * GRU_UPT;
+            const float* rp = s.recv + ((size_t)src * Bp + row) * RW + uh * GRU_UPT;
 #pragma unroll
             for (int gg = 0; gg < 3; ++gg) {
               const float4 a = *reinterpret_cast<const float4*>(rp + gg * GRU_HC);
@@ -1159,50 +1260,14 @@ gru_fwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
         }
       }
       const long long m = (long long)t * Bp + row;
-      float hn[GRU_UPT], rr[GRU_UPT], zz[GRU_UPT], nn[GRU_UPT];
-      if (active) {
-#pragma unroll
-        for (int jj = 0; jj < GRU_UPT; ++jj) {
-          rr[jj] = fast_sigmoid(gi[0][jj] + acc[0][jj] + bias[0][jj]);
-          zz[jj] = fast_sigmoid(gi[1][jj] + acc[1][jj] + bias[1][jj]);
-          hn[jj] = acc[2][jj] + bias[2][jj];
-          nn[jj] = fast_tanh(gi[2][jj] + rr[jj] * hn[jj]);
-          hprev[jj] = (1.f - zz[jj]) * nn[jj] + zz[jj] * hprev[jj];
-        }
-        // critical path: only the bf16 h_t that the other CTAs gather next step
-        *reinterpret_cast<uint4*>(p.xn + m * D + dir * H + ju) = pack8(hprev);
-        if (tid == 0) GRU_STAMP(5);
-        fence_proxy_async_global();   // generic writes -> other CTAs' TMA reads
-        if (tid == 0) GRU_STAMP(6);
-      }
-      epi_barrier();
-      if (tid == 0) {
-        GRU_STAMP(7);
-        if (p.dbg && step == 20) p.dbg[1024 + blockIdx.x] = gtime();         // skew probe
-        grid_arrive(ctr);
-        GRU_STAMP(9);
-      }
-      if (active) {
-        st8(p.y + m * D + dir * H + ju, hprev);
-        if (p.gates) {
-          float* go = p.gates + ((m * p.ndir + dir) * 4) * H + ju;
-          st8(go, rr);
-          st8(go + H, zz);
-          st8(go + 2 * H, nn);
-          st8(go + 3 * H, hn);
-        }
-      }
+      GruGates<GRU_UPT> g;
+      if (active) gru_cell_fwd(gi, acc, bias, hprev, g);
+      gru_publish_fwd(p, step, tid, active, p.xn + m * D + dir * H + ju, hprev, ctr, true);
+      if (active) gru_store_fwd(p, m, dir, ju, hprev, g);
       if (tid == 0) GRU_STAMP(10);
     }
   }
-
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 8) {
-    tc_fence_after_sync();
-    tmem_dealloc(tmem_base, 256);
-  }
+  gru_teardown(tmem_base, 256);
 }
 
 // =============================================================================================
@@ -1224,29 +1289,6 @@ gru_fwd_ks_kernel(const __grid_constant__ CUtensorMap tm_d0,
 // Requires cluster size 4, H % 256 == 0, Bp <= 64 (Bp % 8 == 0 as everywhere).
 // =============================================================================================
 template <int UPT>
-SB_DEVINL void ldu(const float* p, float (&v)[UPT]) {
-  if constexpr (UPT == 2) {
-    const float2 a = __ldcs(reinterpret_cast<const float2*>(p));
-    v[0] = a.x; v[1] = a.y;
-  } else {
-    v[0] = __ldcs(p);
-  }
-}
-template <int UPT>
-SB_DEVINL void stu(float* p, const float (&v)[UPT]) {
-  if constexpr (UPT == 2) __stcs(reinterpret_cast<float2*>(p), make_float2(v[0], v[1]));
-  else __stcs(p, v[0]);
-}
-template <int UPT>
-SB_DEVINL void st_bf16u(bf16* p, const float (&v)[UPT]) {
-  if constexpr (UPT == 2) {
-    *reinterpret_cast<uint32_t*>(p) = pack_bf16x2(v[0], v[1]);
-  } else {
-    *p = __float2bfloat16_rn(v[0]);
-  }
-}
-
-template <int UPT>
 __global__ void __launch_bounds__(GRU_THREADS, 1)
 gru_fwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
                   const __grid_constant__ CUtensorMap tm_d1, const GruFwdParams p) {
@@ -1267,32 +1309,13 @@ gru_fwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
   const int slice = RW * P;                           // floats per (source, owner) slice
   const int NB = (Bp + 15) & ~15;                     // MMA N (rows of h read per chunk)
   const int stride = Bp * 128;
-  const int ring_bytes = nchunks * stride;            // the whole quarter is resident
-  const int wbytes = nchunks * WCHUNK;
-  // carve: ring | weights | recv | stage | barriers.  The N-side read of the last chunk may run
-  // up to 8 rows past the ring into the weights, and the 128-row M-side read of tile 1 runs 64
-  // rows past its 64 valid ones (into the next chunk / the receive buffer): both only feed
-  // accumulator columns / lanes that are never read.
-  uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
-                                             ~static_cast<uintptr_t>(1023));
-  uint8_t* ring = base;
-  uint8_t* wtile = ring + ring_bytes;
-  float* recv = reinterpret_cast<float*>(wtile + wbytes);          // [KS src][48][P]
-  float* stage = recv + KS * slice;                                // [KS-1 dst][48][P]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(stage + (KS - 1) * slice);
-  uint64_t* full = bars;
-  uint64_t* accfull = bars + 1;
-  uint64_t* recvbar = bars + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3);
-  float* bias_s = reinterpret_cast<float*>(bars + 4);             // [48]
+  const GruSmemLayout L = gru_layout_fwd_kt(Bp, H);
+  const GruSmem s = gru_carve(smem_raw, L);           // recv [KS src][48][P], stage [KS-1 dst]
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int D = p.ndir * H;
   const CUtensorMap* tm = dir == 0 ? &tm_d0 : &tm_d1;
 
-  for (int k = tid; k < (ring_bytes + wbytes + (2 * KS - 1) * slice * 4) / 16; k += GRU_THREADS)
-    reinterpret_cast<uint4*>(base)[k] = make_uint4(0, 0, 0, 0);
-  __syncthreads();
-  {
+  const uint32_t tmem_base = gru_setup(s, L, tm, 128, KS, [&] {
     // resident operand: rows ordered by owner (see above), columns = this CTA's K quarter
     const int pieces_per_row = nchunks * 8;
     for (int k = tid; k < WROWS * pieces_per_row; k += GRU_THREADS) {
@@ -1303,27 +1326,13 @@ gru_fwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
       const uint4 v = *reinterpret_cast<const uint4*>(
           p.whh + ((long long)dir * 3 * H + (long long)g * H + k0c + u) * H + (long long)crank * KQ +
           pc * 8);
-      *reinterpret_cast<uint4*>(wtile + (pc >> 3) * WCHUNK + sw128_offset(r, pc & 7)) = v;
+      *reinterpret_cast<uint4*>(s.wtile + (pc >> 3) * WCHUNK + sw128_offset(r, pc & 7)) = v;
     }
     if (tid < RW) {
       const int g = tid / GRU_HC, jj = tid % GRU_HC;
-      bias_s[tid] = p.bhh[dir * 3 * H + g * H + j0 + jj];
+      s.scratch[tid] = p.bhh[dir * 3 * H + g * H + j0 + jj];
     }
-  }
-  if (tid == 0) {
-    mbar_init(full, 1);
-    mbar_init(accfull, 1);
-    mbar_init(recvbar, 1);   // one local arrive.expect_tx per step; the peers' copies complete_tx
-    mbar_fence_init();
-    tma_prefetch_desc(tm);
-  }
-  if (warp == 8) tmem_alloc(tmem_slot, 128);
-  fence_proxy_async_smem();
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  cluster_sync_all();
-  const uint32_t tmem_base = *tmem_slot;
+  });
   unsigned int* ctr = p.barrier + dir * 32;   // one L2 line per direction
 
   if (warp == 9) {
@@ -1335,9 +1344,7 @@ gru_fwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
         grid_wait(ctr, (unsigned int)nC * step);   // all CTAs published h_{tp}
         GRU_STAMP(0);
         if (p.dbg && step == 21) p.dbg[1024 + 256 + blockIdx.x] = gtime();   // skew probe
-        mbar_expect_tx(full, (uint32_t)(stride * nchunks));
-        for (int c = 0; c < nchunks; ++c)
-          tma_load_2d(ring + c * stride, tm, full, (int)crank * KQ + c * 64, tp * Bp);
+        ks_gather_fwd(s, tm, stride, nchunks, (int)crank * KQ, tp * Bp);
         GRU_STAMP(1);
       }
     }
@@ -1346,21 +1353,7 @@ gru_fwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
     if (lane == 0) {
       const uint32_t idesc = umma_idesc_bf16_f32(128, (uint32_t)NB);
       for (int step = 1; step < T; ++step) {
-        mbar_wait(full, (step - 1) & 1);
-        tc_fence_after_sync();
-        for (int c = 0; c < nchunks; ++c) {
-          const uint64_t da0 = umma_desc_sw128_kmajor(smem_u32(wtile + c * WCHUNK));
-          const uint64_t da1 = umma_desc_sw128_kmajor(smem_u32(wtile + c * WCHUNK + 128 * 128));
-          const uint64_t db = umma_desc_sw128_kmajor(smem_u32(ring + c * stride));
-#pragma unroll
-          for (int kk = 0; kk < 4; ++kk) {
-            const uint32_t acc = (c > 0 || kk > 0) ? 1u : 0u;
-            umma_bf16_ss(tmem_base, da0 + (uint64_t)(kk * 2), db + (uint64_t)(kk * 2), idesc, acc);
-            umma_bf16_ss(tmem_base + 64, da1 + (uint64_t)(kk * 2), db + (uint64_t)(kk * 2), idesc,
-                         acc);
-          }
-        }
-        umma_commit(accfull);
+        ks_mma_fwd(s, tmem_base, stride, nchunks, WCHUNK, idesc, true, (step - 1) & 1);
         GRU_STAMP(2);
       }
     }
@@ -1375,8 +1368,8 @@ gru_fwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
     const uint32_t own0 = (uint32_t)sub;                            // owner of the tile-0 row
     const uint32_t own1 = (uint32_t)(sub * 2 + (lane >> 4));        // owner of the tile-1 row
     const uint32_t q0 = (own0 + KS - crank) % KS, q1 = (own1 + KS - crank) % KS;
-    float* dst0 = (q0 == 0 ? recv + crank * slice : stage + (q0 - 1) * slice) + lane * P;
-    float* dst1 = (q1 == 0 ? recv + crank * slice : stage + (q1 - 1) * slice) +
+    float* dst0 = (q0 == 0 ? s.recv + crank * slice : s.stage + (q0 - 1) * slice) + lane * P;
+    float* dst1 = (q1 == 0 ? s.recv + crank * slice : s.stage + (q1 - 1) * slice) +
                   (2 * GRU_HC + (lane & 15)) * P;
     // phase B (gate math): thread = (batch row b, UPT of the CTA's 16 units)
     const int b = tid % Bp, ug = tid / Bp;
@@ -1390,26 +1383,22 @@ gru_fwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
 #pragma unroll
     for (int g = 0; g < 3; ++g)
 #pragma unroll
-      for (int jj = 0; jj < UPT; ++jj) bias[g][jj] = active ? bias_s[g * GRU_HC + u0 + jj] : 0.f;
+      for (int jj = 0; jj < UPT; ++jj) bias[g][jj] = active ? s.scratch[g * GRU_HC + u0 + jj] : 0.f;
 
     for (int step = 0; step < T; ++step) {
       const int t = dir == 0 ? step : (T - 1 - step);
       float gi[3][UPT];
-      if (active) {
-        const float* g = p.gi + ((long long)t * Bp + b) * (p.ndir * 3 * H) + dir * 3 * H + ju;
-#pragma unroll
-        for (int gg = 0; gg < 3; ++gg) ldu<UPT>(g + gg * H, gi[gg]);
-      }
+      if (active) gru_load_gi(p, t, b, dir, ju, gi);
       float acc[3][UPT];
 #pragma unroll
       for (int gg = 0; gg < 3; ++gg)
 #pragma unroll
         for (int jj = 0; jj < UPT; ++jj) acc[gg][jj] = 0.f;
       if (step > 0) {
-        mbar_wait(accfull, (step - 1) & 1);
+        mbar_wait(s.accfull, (step - 1) & 1);
         if (tid == 0) GRU_STAMP(3);
         tc_fence_after_sync();
-        if (tid == 0) mbar_expect_tx(recvbar, (uint32_t)((KS - 1) * slice * 4));
+        if (tid == 0) mbar_expect_tx(s.recvbar, (uint32_t)((KS - 1) * slice * 4));
         {
           const uint32_t tl = tmem_base + ((uint32_t)(sub * 32) << 16) + (uint32_t)(blk0 * 8);
 #pragma unroll
@@ -1449,16 +1438,16 @@ gru_fwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
         epi_barrier();              // all three outgoing slices (and the own one) are staged
         if (lane == 0 && warp >= 1 && warp <= KS - 1) {
           const uint32_t pr = (crank + (uint32_t)warp) % KS;
-          bulk_s2peer(mapa_shared(smem_u32(recv + (size_t)crank * slice), pr),
-                      stage + (size_t)(warp - 1) * slice, (uint32_t)(slice * 4),
-                      mapa_shared(smem_u32(recvbar), pr));
+          bulk_s2peer(mapa_shared(smem_u32(s.recv + (size_t)crank * slice), pr),
+                      s.stage + (size_t)(warp - 1) * slice, (uint32_t)(slice * 4),
+                      mapa_shared(smem_u32(s.recvbar), pr));
         }
         if (tid == 0) GRU_STAMP(4);
-        mbar_wait(recvbar, (step - 1) & 1);
+        mbar_wait(s.recvbar, (step - 1) & 1);
         if (active) {
 #pragma unroll
           for (int src = 0; src < KS; ++src) {
-            const float* rp = recv + (size_t)src * slice + u0 * P + b;
+            const float* rp = s.recv + (size_t)src * slice + u0 * P + b;
 #pragma unroll
             for (int gg = 0; gg < 3; ++gg)
 #pragma unroll
@@ -1467,73 +1456,28 @@ gru_fwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
         }
       }
       const long long m = (long long)t * Bp + b;
-      float hn[UPT], rr[UPT], zz[UPT], nn[UPT];
-      if (active) {
-#pragma unroll
-        for (int jj = 0; jj < UPT; ++jj) {
-          rr[jj] = fast_sigmoid(gi[0][jj] + acc[0][jj] + bias[0][jj]);
-          zz[jj] = fast_sigmoid(gi[1][jj] + acc[1][jj] + bias[1][jj]);
-          hn[jj] = acc[2][jj] + bias[2][jj];
-          nn[jj] = fast_tanh(gi[2][jj] + rr[jj] * hn[jj]);
-          hprev[jj] = (1.f - zz[jj]) * nn[jj] + zz[jj] * hprev[jj];
-        }
-        // critical path: only the bf16 h_t that the other CTAs gather next step
-        st_bf16u<UPT>(p.xn + m * D + dir * H + ju, hprev);
-        if (tid == 0) GRU_STAMP(5);
-        fence_proxy_async_global();   // generic writes -> other CTAs' TMA reads
-        if (tid == 0) GRU_STAMP(6);
-      }
-      epi_barrier();
-      if (tid == 0) {
-        GRU_STAMP(7);
-        if (p.dbg && step == 20) p.dbg[1024 + blockIdx.x] = gtime();         // skew probe
-        grid_arrive(ctr);
-        GRU_STAMP(9);
-      }
-      if (active) {
-        stu<UPT>(p.y + m * D + dir * H + ju, hprev);
-        if (p.gates) {
-          float* go = p.gates + ((m * p.ndir + dir) * 4) * H + ju;
-          stu<UPT>(go, rr);
-          stu<UPT>(go + H, zz);
-          stu<UPT>(go + 2 * H, nn);
-          stu<UPT>(go + 3 * H, hn);
-        }
-      }
+      GruGates<UPT> g;
+      if (active) gru_cell_fwd(gi, acc, bias, hprev, g);
+      gru_publish_fwd(p, step, tid, active, p.xn + m * D + dir * H + ju, hprev, ctr, true);
+      if (active) gru_store_fwd(p, m, dir, ju, hprev, g);
       if (tid == 0) GRU_STAMP(10);
     }
   }
-
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 8) {
-    tc_fence_after_sync();
-    tmem_dealloc(tmem_base, 128);
-  }
+  gru_teardown(tmem_base, 128);
 }
 
 // =============================================================================================
 // backward, K split with the accumulator TRANSPOSED (see gru_fwd_kt_kernel):
 //     D^T[64 units x Bp] = W_hh^T[64 units of the cluster, quarter r of 3H] * dgh[:, quarter r]^T
-// The weight tile is the one of gru_bwd_ks_kernel (its 64 rows are already grouped by owner:
-// rows 16q..16q+15 belong to CTA q of the cluster); an accumulator lane is a unit, so its row
-// of Bp partial sums goes to exactly one peer, and the elementwise work runs on all 256
-// epilogue threads (thread = batch row x UPT units).
+// The weight tile is the one of gru_bwd_ks_kernel (its 64 rows are already grouped by owner);
+// an accumulator lane is a unit, so its row of Bp partial sums goes to exactly one peer, and the
+// elementwise work runs on all 256 epilogue threads (thread = batch row x 1 unit; the 128-row
+// M-side read covers the next weight chunk with its lanes 64..127, which are never read).
 // =============================================================================================
-template <int UPT>
-SB_DEVINL void st_stream_bf16u(bf16* p, const float (&v)[UPT]) {
-  if constexpr (UPT == 2) {
-    __stcs(reinterpret_cast<unsigned int*>(p), pack_bf16x2(v[0], v[1]));
-  } else {
-    st_stream_bf16(p, v[0]);
-  }
-}
-
-template <int UPT>
 __global__ void __launch_bounds__(GRU_THREADS, 1)
 gru_bwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
                   const __grid_constant__ CUtensorMap tm_d1, const GruBwdParams p) {
+  constexpr int UPT = 1;
   extern __shared__ uint8_t smem_raw[];
   const int H = p.H, Bp = p.Bp, T = p.T;
   const int nC = H / GRU_HC;
@@ -1545,68 +1489,19 @@ gru_bwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
   const int K3 = 3 * H;
   const int KQ = K3 / KS;                             // this CTA's share of the contraction
   const int nchunks = KQ / 64;
-  constexpr int WCHUNK = 64 * 128;                    // 64 rows (units) x 64 bf16
   const int P = Bp + 4;                               // pitch of a staged row (floats)
   const int slice = GRU_HC * P;                       // floats per (source, owner) slice
   const int NB = (Bp + 15) & ~15;
   const int stride = Bp * 128;
-  const int ring_bytes = nchunks * stride;            // the whole quarter is resident
-  const int wbytes = nchunks * WCHUNK;
-  // carve: ring | weights | recv | stage | barriers.  The 128-row M-side read covers the next
-  // weight chunk (last chunk: the receive buffer) with its lanes 64..127, which are never read.
-  uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
-                                             ~static_cast<uintptr_t>(1023));
-  uint8_t* ring = base;
-  uint8_t* wtile = ring + ring_bytes;
-  float* recv = reinterpret_cast<float*>(wtile + wbytes);          // [KS src][16][P]
-  float* stage = recv + KS * slice;                                // [KS-1 dst][16][P]
-  float* pad_end = stage + (KS - 1) * slice;
-  // the last chunk's 128-row read needs 8 KB after the weights: recv + stage cover it only for
-  // large batches, so reserve it explicitly
-  const int tail_floats = max(0, 2048 - (2 * KS - 1) * slice);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(pad_end + tail_floats);
-  uint64_t* full = bars;          // [4] groups
-  uint64_t* accfull = bars + 4;
-  uint64_t* recvbar = bars + 5;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 6);
+  const GruSmemLayout L = gru_layout_bwd_kt(Bp, H);
+  const GruSmem s = gru_carve(smem_raw, L);           // recv [KS src][16][P], stage [KS-1 dst]
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int D = p.ndir * H;
   const CUtensorMap* tm = dir == 0 ? &tm_d0 : &tm_d1;
-  const int gc = (nchunks % 4 == 0) ? 4 : ((nchunks % 3 == 0) ? 3 : ((nchunks % 2 == 0) ? 2 : 1));
-  const int ngroups = nchunks / gc;                   // <= 4 for H <= 1024 ... checked on host
+  const int gc = gru_group_chunks(nchunks);
+  const int ngroups = nchunks / gc;                   // <= GRU_KS_BWD_GROUPS: checked on the host
 
-  for (int k = tid; k < (ring_bytes + wbytes + ((2 * KS - 1) * slice + tail_floats) * 4) / 16;
-       k += GRU_THREADS)
-    reinterpret_cast<uint4*>(base)[k] = make_uint4(0, 0, 0, 0);
-  __syncthreads();
-  {
-    // resident operand: see gru_bwd_ks_kernel
-    for (int k = tid; k < KQ * 8; k += GRU_THREADS) {
-      const int kl = k >> 3, piece = k & 7;       // local k, 8-unit piece of the 64 units
-      const uint4 v = *reinterpret_cast<const uint4*>(
-          p.whh + ((long long)dir * K3 + (long long)crank * KQ + kl) * H + k0c + piece * 8);
-      const unsigned short* e = reinterpret_cast<const unsigned short*>(&v);
-      uint8_t* chunk = wtile + (kl >> 6) * WCHUNK + (kl & 7) * 2;
-#pragma unroll
-      for (int q = 0; q < 8; ++q)
-        *reinterpret_cast<unsigned short*>(
-            chunk + sw128_offset((uint32_t)(piece * 8 + q), (uint32_t)((kl & 63) >> 3))) = e[q];
-    }
-  }
-  if (tid == 0) {
-    for (int i = 0; i < 4; ++i) mbar_init(&full[i], 1);
-    mbar_init(accfull, 1);
-    mbar_init(recvbar, 1);
-    mbar_fence_init();
-    tma_prefetch_desc(tm);
-  }
-  if (warp == 8) tmem_alloc(tmem_slot, 64);
-  fence_proxy_async_smem();
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  cluster_sync_all();
-  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_base =
+      gru_setup(s, L, tm, 64, KS, [&] { ks_stage_whh_t(s.wtile, p.whh, H, dir, k0c, crank); });
   unsigned int* ctr = p.barrier + dir * 32;   // one L2 line per direction
 
   if (warp == 9) {
@@ -1614,14 +1509,7 @@ gru_bwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
       for (int step = 0; step + 1 < T; ++step) {
         grid_wait(ctr, (unsigned int)nC * (step + 1));   // dgh of this step is complete
         GRU_STAMP(0);
-        for (int g = 0; g < ngroups; ++g) {
-          mbar_expect_tx(&full[g], (uint32_t)(stride * gc));
-          for (int i = 0; i < gc; ++i) {
-            const int c = g * gc + i;
-            tma_load_2d(ring + c * stride, tm, &full[g], (int)crank * KQ + c * 64,
-                        (step & 1) * Bp);
-          }
-        }
+        ks_gather_bwd(s, tm, stride, ngroups, gc, (int)crank * KQ, (step & 1) * Bp);
         GRU_STAMP(1);
       }
     }
@@ -1629,20 +1517,7 @@ gru_bwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
     if (lane == 0) {
       const uint32_t idesc = umma_idesc_bf16_f32(128, (uint32_t)NB);
       for (int step = 0; step + 1 < T; ++step) {
-        for (int g = 0; g < ngroups; ++g) {
-          mbar_wait(&full[g], step & 1);
-          tc_fence_after_sync();
-          for (int i = 0; i < gc; ++i) {
-            const int c = g * gc + i;
-            const uint64_t da = umma_desc_sw128_kmajor(smem_u32(wtile + c * WCHUNK));
-            const uint64_t db = umma_desc_sw128_kmajor(smem_u32(ring + c * stride));
-#pragma unroll
-            for (int kk = 0; kk < 4; ++kk)
-              umma_bf16_ss(tmem_base, da + (uint64_t)(kk * 2), db + (uint64_t)(kk * 2), idesc,
-                           (c > 0 || kk > 0) ? 1u : 0u);
-          }
-        }
-        umma_commit(accfull);
+        ks_mma_bwd(s, tmem_base, stride, ngroups, gc, 64 * 128, idesc, true, step & 1);
         GRU_STAMP(2);
       }
     }
@@ -1654,17 +1529,18 @@ gru_bwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
     const int myblk = hi == 0 ? (nblk + 1) / 2 : nblk / 2;          // <= 4
     const uint32_t own = (uint32_t)(sub * 2 + (lane >> 4));
     const uint32_t q0 = (own + KS - crank) % KS;
-    float* dst0 = (q0 == 0 ? recv + crank * slice : stage + (q0 - 1) * slice) + (lane & 15) * P;
-    // phase B: thread = (batch row b, UPT of the CTA's 16 units)
+    float* dst0 =
+        (q0 == 0 ? s.recv + crank * slice : s.stage + (q0 - 1) * slice) + (lane & 15) * P;
+    // phase B: thread = (batch row b, one of the CTA's 16 units)
     const int b = tid % Bp, ug = tid / Bp;
     const bool active = ug * UPT < GRU_HC;
     const int u0 = ug * UPT;
     const int ju = j0 + u0;
     float dh_rec[UPT];
-    float db_r[UPT], db_z[UPT], db_n[UPT], db_hn[UPT];
+    GruGrad<UPT> db;
 #pragma unroll
     for (int jj = 0; jj < UPT; ++jj) {
-      dh_rec[jj] = 0.f; db_r[jj] = 0.f; db_z[jj] = 0.f; db_n[jj] = 0.f; db_hn[jj] = 0.f;
+      dh_rec[jj] = 0.f; db.r[jj] = 0.f; db.z[jj] = 0.f; db.n[jj] = 0.f; db.nr[jj] = 0.f;
     }
 
     for (int step = 0; step < T; ++step) {
@@ -1673,26 +1549,14 @@ gru_bwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
       const bool has_prev = dir == 0 ? (t > 0) : (t < T - 1);
       bf16* xb = p.xchg + ((long long)(dir * 2 + (step & 1)) * Bp) * K3;
       const long long m = (long long)t * Bp + b;
-      float rr[UPT], zz[UPT], nn[UPT], hn[UPT], dh[UPT], hp[UPT];
-      if (active) {
-        const float* go = p.gates + ((m * p.ndir + dir) * 4) * H + ju;
-        ldu<UPT>(go, rr);
-        ldu<UPT>(go + H, zz);
-        ldu<UPT>(go + 2 * H, nn);
-        ldu<UPT>(go + 3 * H, hn);
-        ldu<UPT>(p.dy + m * D + dir * H + ju, dh);
-        if (has_prev) {
-          ldu<UPT>(p.y + ((long long)tp * Bp + b) * D + dir * H + ju, hp);
-        } else {
-#pragma unroll
-          for (int jj = 0; jj < UPT; ++jj) hp[jj] = 0.f;
-        }
-      }
+      GruGates<UPT> a;
+      float dh[UPT], hp[UPT];
+      if (active) gru_load_bwd(p, m, (long long)tp * Bp + b, has_prev, dir, ju, a, dh, hp);
       if (step > 0) {
-        mbar_wait(accfull, (step - 1) & 1);
+        mbar_wait(s.accfull, (step - 1) & 1);
         if (tid == 0) GRU_STAMP(3);
         tc_fence_after_sync();
-        if (tid == 0) mbar_expect_tx(recvbar, (uint32_t)((KS - 1) * slice * 4));
+        if (tid == 0) mbar_expect_tx(s.recvbar, (uint32_t)((KS - 1) * slice * 4));
         if (sub < 2) {
           const uint32_t tl = tmem_base + ((uint32_t)(sub * 32) << 16) + (uint32_t)(blk0 * 8);
           uint32_t v[4][8];
@@ -1716,116 +1580,65 @@ gru_bwd_kt_kernel(const __grid_constant__ CUtensorMap tm_d0,
         epi_barrier();
         if (lane == 0 && warp >= 1 && warp <= KS - 1) {
           const uint32_t pr = (crank + (uint32_t)warp) % KS;
-          bulk_s2peer(mapa_shared(smem_u32(recv + (size_t)crank * slice), pr),
-                      stage + (size_t)(warp - 1) * slice, (uint32_t)(slice * 4),
-                      mapa_shared(smem_u32(recvbar), pr));
+          bulk_s2peer(mapa_shared(smem_u32(s.recv + (size_t)crank * slice), pr),
+                      s.stage + (size_t)(warp - 1) * slice, (uint32_t)(slice * 4),
+                      mapa_shared(smem_u32(s.recvbar), pr));
         }
         if (tid == 0) GRU_STAMP(4);
-        mbar_wait(recvbar, (step - 1) & 1);
+        mbar_wait(s.recvbar, (step - 1) & 1);
         if (active) {
 #pragma unroll
           for (int src = 0; src < KS; ++src) {
-            const float* rp = recv + (size_t)src * slice + u0 * P + b;
+            const float* rp = s.recv + (size_t)src * slice + u0 * P + b;
 #pragma unroll
             for (int jj = 0; jj < UPT; ++jj) dh_rec[jj] += rp[jj * P];
           }
         }
       }
-      float dr[UPT], dz[UPT], dn[UPT], dnr[UPT];
-      if (active) {
-#pragma unroll
-        for (int jj = 0; jj < UPT; ++jj) {
-          const float g = dh[jj] + dh_rec[jj];
-          dn[jj] = g * (1.f - zz[jj]) * (1.f - nn[jj] * nn[jj]);
-          dz[jj] = g * (hp[jj] - nn[jj]) * zz[jj] * (1.f - zz[jj]);
-          dr[jj] = dn[jj] * hn[jj] * rr[jj] * (1.f - rr[jj]);
-          dnr[jj] = dn[jj] * rr[jj];
-          dh_rec[jj] = g * zz[jj];
-          db_r[jj] += dr[jj];
-          db_z[jj] += dz[jj];
-          db_n[jj] += dn[jj];
-          db_hn[jj] += dnr[jj];
-        }
-        if (step + 1 < T) {
-          bf16* x = xb + (long long)b * K3 + ju;
-          st_bf16u<UPT>(x, dr);
-          st_bf16u<UPT>(x + H, dz);
-          st_bf16u<UPT>(x + 2 * H, dnr);
-          if (tid == 0) GRU_STAMP(5);
-          fence_proxy_async_global();
-          if (tid == 0) GRU_STAMP(6);
-        }
-      }
-      if (step + 1 < T) {
-        epi_barrier();
-        if (tid == 0) {
-          GRU_STAMP(7);
-          grid_arrive(ctr);
-          GRU_STAMP(9);
-        }
-      }
-      if (active) {
-        bf16* o = p.dgi + m * (p.ndir * K3) + dir * K3 + ju;
-        st_stream_bf16u<UPT>(o, dr);
-        st_stream_bf16u<UPT>(o + H, dz);
-        st_stream_bf16u<UPT>(o + 2 * H, dn);
-        st_stream_bf16u<UPT>(p.dghn + m * D + dir * H + ju, dnr);
-      }
+      GruGrad<UPT> d;
+      if (active) gru_cell_bwd(a, dh, hp, dh_rec, d, db);
+      gru_publish_bwd(p, step, tid, active, xb + (long long)b * K3 + ju, d, ctr);
+      if (active) gru_store_bwd(p, m, dir, ju, d);
       if (tid == 0) GRU_STAMP(10);
     }
     if (active) {
 #pragma unroll
       for (int jj = 0; jj < UPT; ++jj) {
         const int bi = dir * K3 + ju + jj;
-        atomicAdd(p.dbih + bi, db_r[jj]);
-        atomicAdd(p.dbih + bi + H, db_z[jj]);
-        atomicAdd(p.dbih + bi + 2 * H, db_n[jj]);
-        atomicAdd(p.dbhh + bi, db_r[jj]);
-        atomicAdd(p.dbhh + bi + H, db_z[jj]);
-        atomicAdd(p.dbhh + bi + 2 * H, db_hn[jj]);
+        atomicAdd(p.dbih + bi, db.r[jj]);
+        atomicAdd(p.dbih + bi + H, db.z[jj]);
+        atomicAdd(p.dbih + bi + 2 * H, db.n[jj]);
+        atomicAdd(p.dbhh + bi, db.r[jj]);
+        atomicAdd(p.dbhh + bi + H, db.z[jj]);
+        atomicAdd(p.dbhh + bi + 2 * H, db.nr[jj]);
       }
     }
   }
-
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 8) {
-    tc_fence_after_sync();
-    tmem_dealloc(tmem_base, 64);
-  }
+  gru_teardown(tmem_base, 64);
 }
 
 int make_tmap_bf16_2d(CUtensorMap* map, const void* base, long long rows, long long cols,
                       long long ld, int box_rows);
 
-// chunks are grouped gc per mbarrier pair (gc = largest of 4,3,2,1 dividing nchunks); ring = the
-// largest divisor of ngroups (<= GRU_MAX_RING) whose slots fit next to the resident weights
-static int gru_ring_slots(int wbytes, int Bp, int nchunks, int* gc_out, size_t* smem_bytes) {
-  int gc = 1;
-  for (int g = 4; g >= 1; --g)
-    if (nchunks % g == 0) { gc = g; break; }
-  const int ngroups = nchunks / gc;
-  const int slot = gc * Bp * 128;
-  const int fixed = wbytes + 1024 /*align*/ + (2 * GRU_MAX_RING + 2) * 8 + 256 /*scratch*/ + 64;
-  int fit = (227 * 1024 - fixed) / slot;
-  if (fit > GRU_MAX_RING) fit = GRU_MAX_RING;
-  int ring = -1;
-  for (int r = fit; r >= 1; --r)
-    if (ngroups % r == 0) { ring = r; break; }
-  if (ring < 1) {
-    if (gc == 1) return -1;
-    // fall back to single-chunk groups
-    gc = 1;
-    fit = (227 * 1024 - fixed) / (Bp * 128);
-    if (fit > GRU_MAX_RING) fit = GRU_MAX_RING;
-    for (int r = fit; r >= 1; --r)
-      if (nchunks % r == 0) { ring = r; break; }
-    if (ring < 1) return -1;
+static constexpr int GRU_SMEM_MAX = 227 * 1024;   // dynamic shared memory of one sm_100 CTA
+
+// chunks are grouped gc per mbarrier pair (gc = largest of 4,3,2,1 dividing nchunks, or 1 when
+// that leaves no ring); ring = the largest divisor of ngroups (<= GRU_MAX_RING) whose slots fit
+// next to the resident weights
+static int gru_ring_slots(int Bp, int nchunks, int wrows, int* gc_out, size_t* smem_bytes) {
+  const int fixed = gru_layout_full(Bp, nchunks, wrows, 0).bytes;
+  for (int gc : {gru_group_chunks(nchunks), 1}) {
+    const int ngroups = nchunks / gc;
+    const int fit = std::min((GRU_SMEM_MAX - fixed) / (gc * Bp * 128), GRU_MAX_RING);
+    for (int r = fit; r >= 1; --r) {
+      if (ngroups % r == 0) {
+        *gc_out = gc;
+        *smem_bytes = (size_t)gru_layout_full(Bp, nchunks, wrows, r * gc * Bp * 128).bytes;
+        return r;
+      }
+    }
   }
-  *gc_out = gc;
-  *smem_bytes = (size_t)fixed + (size_t)ring * gc * Bp * 128;
-  return ring;
+  return -1;
 }
 
 static int g_gru_last_cluster = 0;
@@ -1889,6 +1702,19 @@ static int gru_launch(const void* kernel, int grid, int nC, int cs_pref, int cs_
   return SB_ERR_UNSUPPORTED;
 }
 
+// The tensor maps of the gathered operand, one per direction (direction 1 aliases direction 0
+// when the layer is unidirectional): `rows` x `cols` bf16 with leading dimension `ld`, the
+// direction's block starting `dir_stride` elements after the previous one, boxes of Bp rows.
+static int gru_tmaps(CUtensorMap (&tm)[2], const bf16* base, long long rows, long long cols,
+                     long long ld, size_t dir_stride, int ndir, int Bp) {
+  for (int d = 0; d < 2; ++d) {
+    const int rc = make_tmap_bf16_2d(&tm[d], base + (d < ndir ? d : 0) * dir_stride, rows, cols,
+                                     ld, Bp);
+    if (rc != SB_OK) return rc;
+  }
+  return SB_OK;
+}
+
 // workspace of one recurrence launch: [0,1024) the per-direction grid-barrier words, then the
 // exchange buffers of the backward kernels
 static constexpr size_t GRU_WS_COUNTERS = 1024;
@@ -1913,6 +1739,20 @@ static int gru_check(int T, int Bp, int H, int ndir) {
   return SB_OK;
 }
 
+// Common to sb_gru_fwd and sb_gru_bwd: validate the shape and the arguments, check the workspace
+// (`need` bytes, 1024-aligned) and zero it: the grid-barrier counters start at 0, and so do the
+// exchange tiles (columns past 3H of a partial chunk are never written and must read as zero).
+static int gru_begin(int T, int Bp, int H, int ndir, bool args_ok, void* workspace,
+                     size_t workspace_bytes, size_t need, cudaStream_t stream) {
+  const int rc = gru_check(T, Bp, H, ndir);
+  if (rc != SB_OK) return rc;
+  if (!args_ok || !workspace) return SB_ERR_INVALID;
+  if (workspace_bytes < need) return SB_ERR_WORKSPACE;
+  if ((reinterpret_cast<uintptr_t>(workspace) & 1023) != 0) return SB_ERR_INVALID;
+  if (cudaMemsetAsync(workspace, 0, need, stream) != cudaSuccess) return SB_ERR_CUDA;
+  return SB_OK;
+}
+
 extern "C" int sb_gru_fwd_workspace_size(int Bp, int H, int ndir, size_t* bytes) {
   if (!bytes || Bp <= 0 || H <= 0 || (ndir != 1 && ndir != 2)) return SB_ERR_INVALID;
   (void)Bp;
@@ -1920,76 +1760,54 @@ extern "C" int sb_gru_fwd_workspace_size(int Bp, int H, int ndir, size_t* bytes)
   return SB_OK;
 }
 
+// Forward kernel selection: the K split over 4-CTA clusters (H % 256 == 0, batch rows <= 64) when
+// its layout fits, kt rather than ks when gru_use_kt picks it and kt fits too; otherwise, or when a
+// K-split grid cannot be co-resident, every CTA gathers all of h_{t-1} (TMA, cluster multicast).
+static int gru_fwd_select(GruFwdParams& p, void** args, cudaStream_t stream) {
+  const int H = p.H, Bp = p.Bp, grid = p.ndir * (H / GRU_HC), nC = H / GRU_HC;
+  int gc = 1;
+  size_t smem = 0;
+  const int ring = gru_ring_slots(Bp, (H + 63) / 64, 48, &gc, &smem);
+  if (ring < 0) return SB_ERR_UNSUPPORTED;
+  if (H % 256 == 0 && Bp <= 64) {
+    const GruSmemLayout ks = gru_layout_fwd_ks(Bp, H), kt = gru_layout_fwd_kt(Bp, H);
+    if (ks.bytes <= GRU_SMEM_MAX) {
+      p.ring = H / KS / 64;
+      p.gc = 1;
+      if (gru_use_kt(Bp, false) && kt.bytes <= GRU_SMEM_MAX) {
+        const void* k = Bp > 16 ? (const void*)gru_fwd_kt_kernel<2> : (const void*)gru_fwd_kt_kernel<1>;
+        if (gru_launch(k, grid, nC, KS, KS, kt.bytes, args, stream) == SB_OK) return SB_OK;
+      }
+      if (gru_launch((const void*)gru_fwd_ks_kernel, grid, nC, KS, KS, ks.bytes, args, stream) ==
+          SB_OK)
+        return SB_OK;
+    }
+  }
+  p.ring = ring;
+  p.gc = gc;
+  return gru_launch((const void*)gru_fwd_kernel, grid, nC, 4, 1, smem, args, stream);
+}
+
 extern "C" int sb_gru_fwd(const float* gi, const void* whh_bf16, const float* bhh, float* y,
                           void* xn_bf16, float* gates, void* workspace, size_t workspace_bytes,
                           int T, int Bp, int H, int ndir, void* stream_) {
-  int rc = gru_check(T, Bp, H, ndir);
-  if (rc != SB_OK) return rc;
-  if (!gi || !whh_bf16 || !bhh || !y || !xn_bf16 || !workspace) return SB_ERR_INVALID;
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   size_t need = 0;
   sb_gru_fwd_workspace_size(Bp, H, ndir, &need);
-  if (workspace_bytes < need) return SB_ERR_WORKSPACE;
-  if ((reinterpret_cast<uintptr_t>(workspace) & 1023) != 0) return SB_ERR_INVALID;
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  const int nchunks = (H + 63) / 64;
-  const int nC = H / GRU_HC;
-  if (cudaMemsetAsync(workspace, 0, need, stream) != cudaSuccess) return SB_ERR_CUDA;
-  uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
-  unsigned int* barrier = reinterpret_cast<unsigned int*>(ws);
-  int gc = 1;
-  size_t smem = 0;
-  const int ring =
-      gru_ring_slots(std::max(nchunks * 48 * 128, 16384 - Bp * 128), Bp, nchunks, &gc, &smem);
-  if (ring < 0) return SB_ERR_UNSUPPORTED;
-
-  // ---- preferred: K-split over 4-CTA clusters (H % 256 == 0, batch rows <= 64) ----
-  if (H % 256 == 0 && nC % KS == 0 && Bp <= 64) {
-    const int nq = H / KS / 64;
-    const size_t ks_smem = (size_t)nq * Bp * 128 + (size_t)nq * 192 * 128 +
-                           (size_t)2 * KS * Bp * 48 * 4 + 1024 + 512;
-    if (ks_smem <= 227 * 1024) {
-      GruFwdParams q;
-      q.gi = gi; q.whh = reinterpret_cast<const bf16*>(whh_bf16); q.bhh = bhh; q.y = y;
-      q.xn = reinterpret_cast<bf16*>(xn_bf16); q.gates = gates;
-      q.barrier = barrier; q.T = T; q.Bp = Bp; q.H = H; q.ndir = ndir;
-      q.dbg = g_gru_dbg; q.ring = nq; q.gc = 1;
-      CUtensorMap tq[2];
-      for (int d = 0; d < 2; ++d) {
-        const int dd = d < ndir ? d : 0;
-        rc = make_tmap_bf16_2d(&tq[d], q.xn + (size_t)dd * H, (long long)T * Bp, H,
-                               (long long)ndir * H, Bp);
-        if (rc != SB_OK) return rc;
-      }
-      void* kargs[] = {(void*)&tq[0], (void*)&tq[1], (void*)&q};
-      const size_t kt_smem = (size_t)nq * Bp * 128 + (size_t)nq * 192 * 128 +
-                             (size_t)(2 * KS - 1) * 48 * (Bp + 4) * 4 + 1024 + 512;
-      if (gru_use_kt(Bp, false) && kt_smem <= 227 * 1024) {
-        const void* kt = Bp > 16 ? (const void*)gru_fwd_kt_kernel<2>
-                                 : (const void*)gru_fwd_kt_kernel<1>;
-        rc = gru_launch(kt, ndir * nC, nC, KS, KS, kt_smem, kargs, stream);
-        if (rc == SB_OK) return SB_OK;
-      }
-      rc = gru_launch((const void*)gru_fwd_ks_kernel, ndir * nC, nC, KS, KS, ks_smem, kargs, stream);
-      if (rc == SB_OK) return SB_OK;
-    }
-  }
-
-  // ---- every other shape: each CTA gathers all of h_{t-1} (tensor-map TMA, cluster multicast) ----
+  int rc = gru_begin(T, Bp, H, ndir, gi && whh_bf16 && bhh && y && xn_bf16, workspace,
+                     workspace_bytes, need, stream);
+  if (rc != SB_OK) return rc;
   GruFwdParams p;
   p.gi = gi; p.whh = reinterpret_cast<const bf16*>(whh_bf16); p.bhh = bhh; p.y = y;
   p.xn = reinterpret_cast<bf16*>(xn_bf16);
-  p.gates = gates; p.barrier = barrier; p.T = T; p.Bp = Bp; p.H = H; p.ndir = ndir;
+  p.gates = gates; p.barrier = reinterpret_cast<unsigned int*>(workspace);
+  p.T = T; p.Bp = Bp; p.H = H; p.ndir = ndir;
   p.dbg = g_gru_dbg;
-  p.ring = ring; p.gc = gc;
   CUtensorMap tm[2];
-  for (int d = 0; d < 2; ++d) {
-    const int dd = d < ndir ? d : 0;
-    rc = make_tmap_bf16_2d(&tm[d], p.xn + (size_t)dd * H, (long long)T * Bp, H,
-                           (long long)ndir * H, Bp);
-    if (rc != SB_OK) return rc;
-  }
+  rc = gru_tmaps(tm, p.xn, (long long)T * Bp, H, (long long)ndir * H, (size_t)H, ndir, Bp);
+  if (rc != SB_OK) return rc;
   void* args[] = {(void*)&tm[0], (void*)&tm[1], (void*)&p};
-  return gru_launch((const void*)gru_fwd_kernel, ndir * nC, nC, 4, 1, smem, args, stream);
+  return gru_fwd_select(p, args, stream);
 }
 
 extern "C" int sb_gru_bwd_workspace_size(int Bp, int H, int ndir, size_t* bytes) {
@@ -2001,20 +1819,44 @@ extern "C" int sb_gru_bwd_workspace_size(int Bp, int H, int ndir, size_t* bytes)
   return SB_OK;
 }
 
+// Backward kernel selection, the chain of the forward one: the K split when its chunk groups fit
+// its full barriers and its layout fits (kt rather than ks when gru_use_kt picks it and kt fits
+// too), otherwise the full gather.
+static int gru_bwd_select(GruBwdParams& p, void** args, cudaStream_t stream) {
+  const int H = p.H, Bp = p.Bp, grid = p.ndir * (H / GRU_HC), nC = H / GRU_HC;
+  const int nchunks = (3 * H + 63) / 64;
+  if (H % 256 == 0) {
+    const GruSmemLayout ks = gru_layout_bwd_ks(Bp, H), kt = gru_layout_bwd_kt(Bp, H);
+    const int nq = 3 * H / KS / 64;
+    if (nq / gru_group_chunks(nq) <= ks.nfull && ks.bytes <= GRU_SMEM_MAX) {
+      p.ring = nq;
+      p.gc = 1;
+      if (gru_use_kt(Bp, true) && kt.bytes <= GRU_SMEM_MAX &&
+          gru_launch((const void*)gru_bwd_kt_kernel, grid, nC, KS, KS, kt.bytes, args, stream) ==
+              SB_OK)
+        return SB_OK;
+      if (gru_launch((const void*)gru_bwd_ks_kernel, grid, nC, KS, KS, ks.bytes, args, stream) ==
+          SB_OK)
+        return SB_OK;
+    }
+  }
+  size_t smem = 0;
+  p.ring = gru_ring_slots(Bp, nchunks, 16, &p.gc, &smem);
+  if (p.ring < 0) return SB_ERR_UNSUPPORTED;
+  return gru_launch((const void*)gru_bwd_kernel, grid, nC, 4, 1, smem, args, stream);
+}
+
 extern "C" int sb_gru_bwd(const float* dy, const float* y, const float* gates,
                           const void* whh_bf16, void* dgi_bf16, void* dghn_bf16, float* dbih,
                           float* dbhh, void* workspace, size_t workspace_bytes, int T, int Bp,
                           int H, int ndir, void* stream_) {
-  int rc = gru_check(T, Bp, H, ndir);
-  if (rc != SB_OK) return rc;
-  if (!dy || !y || !gates || !whh_bf16 || !dgi_bf16 || !dghn_bf16 || !dbih || !dbhh ||
-      !workspace)
-    return SB_ERR_INVALID;
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   size_t need = 0;
   sb_gru_bwd_workspace_size(Bp, H, ndir, &need);
-  if (workspace_bytes < need) return SB_ERR_WORKSPACE;
-  if ((reinterpret_cast<uintptr_t>(workspace) & 1023) != 0) return SB_ERR_INVALID;
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  int rc = gru_begin(T, Bp, H, ndir,
+                     dy && y && gates && whh_bf16 && dgi_bf16 && dghn_bf16 && dbih && dbhh,
+                     workspace, workspace_bytes, need, stream);
+  if (rc != SB_OK) return rc;
   uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
   GruBwdParams p;
   p.dy = dy; p.y = y; p.gates = gates; p.whh = reinterpret_cast<const bf16*>(whh_bf16);
@@ -2024,49 +1866,11 @@ extern "C" int sb_gru_bwd(const float* dy, const float* y, const float* gates,
   p.xchg = reinterpret_cast<bf16*>(ws + GRU_WS_COUNTERS);
   p.dbih = dbih; p.dbhh = dbhh; p.T = T; p.Bp = Bp; p.H = H; p.ndir = ndir;
   p.dbg = g_gru_dbg;
-  const int K3 = 3 * H;
-  const int nchunks = (K3 + 63) / 64;
-  size_t smem = 0;
-  const int nC_ = H / GRU_HC;
-  // counters and barrier words start at zero; the exchange tiles too (columns past 3H of a
-  // partial chunk are never written and must read as zero)
-  if (cudaMemsetAsync(workspace, 0, need, stream) != cudaSuccess) return SB_ERR_CUDA;
-  // ---- preferred: K-split over 4-CTA clusters ----
-  if (H % 256 == 0 && nC_ % KS == 0 && (K3 / KS / 64) <= 16) {
-    const int nq = K3 / KS / 64;
-    const size_t ks_smem = (size_t)nq * Bp * 128 + (size_t)nq * 64 * 128 +
-                           (size_t)2 * KS * Bp * 64 + 1024 + 256;
-    if (ks_smem <= 227 * 1024) {
-      CUtensorMap tq[2];
-      for (int d = 0; d < 2; ++d) {
-        const int dd = d < ndir ? d : 0;
-        rc = make_tmap_bf16_2d(&tq[d], p.xchg + (size_t)dd * 2 * Bp * K3, 2LL * Bp, K3, K3, Bp);
-        if (rc != SB_OK) return rc;
-      }
-      p.ring = nq; p.gc = 1;
-      void* kargs[] = {(void*)&tq[0], (void*)&tq[1], (void*)&p};
-      const size_t ex = (size_t)(2 * KS - 1) * GRU_HC * (Bp + 4) * 4;
-      const size_t kt_smem = (size_t)nq * Bp * 128 + (size_t)nq * 64 * 128 +
-                             std::max(ex, (size_t)8192) + 1024 + 256;
-      if (gru_use_kt(Bp, true) && kt_smem <= 227 * 1024) {
-        rc = gru_launch((const void*)gru_bwd_kt_kernel<1>, ndir * nC_, nC_, KS, KS, kt_smem, kargs,
-                        stream);
-        if (rc == SB_OK) return SB_OK;
-      }
-      rc = gru_launch((const void*)gru_bwd_ks_kernel, ndir * nC_, nC_, KS, KS, ks_smem, kargs,
-                      stream);
-      if (rc == SB_OK) return SB_OK;
-    }
-  }
-  p.ring = gru_ring_slots(std::max(nchunks * 16 * 128, 16384 - Bp * 128), Bp, nchunks, &p.gc, &smem);
-  if (p.ring < 0) return SB_ERR_UNSUPPORTED;
   // per direction: the two parity buffers stacked as [2*Bp rows][3H cols]
+  const int K3 = 3 * H;
   CUtensorMap tm[2];
-  for (int d = 0; d < 2; ++d) {
-    const int dd = d < ndir ? d : 0;
-    rc = make_tmap_bf16_2d(&tm[d], p.xchg + (size_t)dd * 2 * Bp * K3, 2LL * Bp, K3, K3, Bp);
-    if (rc != SB_OK) return rc;
-  }
+  rc = gru_tmaps(tm, p.xchg, 2LL * Bp, K3, K3, (size_t)2 * Bp * K3, ndir, Bp);
+  if (rc != SB_OK) return rc;
   void* args[] = {(void*)&tm[0], (void*)&tm[1], (void*)&p};
-  return gru_launch((const void*)gru_bwd_kernel, ndir * nC_, nC_, 4, 1, smem, args, stream);
+  return gru_bwd_select(p, args, stream);
 }

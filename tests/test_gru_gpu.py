@@ -37,6 +37,10 @@ def _ref_and_ours(B, T, In, H, L, bidir, seed):
     (3, 9, 40, 32, 2, True),       # ragged batch (padded to 8), 2 layers bi
     (8, 20, 64, 128, 2, True),     # several CTAs per direction
     (16, 31, 480, 256, 3, True),   # shipped-config width
+    # uni H = 1280: the backward K split would need 5 chunk groups of its 4 full barriers, so the
+    # backward must take the full gather at 8 and 16 rows, where kt / ks would otherwise be picked
+    (8, 5, 64, 1280, 1, False),
+    (16, 5, 64, 1280, 1, False),
 ])
 def test_gru_stack_forward_backward(cuda_lib, B, T, In, H, L, bidir):
     rnn64, x64, y64, rnn_c, xc, yc = _ref_and_ours(B, T, In, H, L, bidir, seed=B + T + H)
